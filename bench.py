@@ -2,6 +2,7 @@
 """Benchmark of the structured-layer hot path (BASELINE.json metric: structured-layer fwd+bwd samples/s).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload sss|lr|lr_bf16|psm|psm_sparse|hmat|ldr] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 A "step" is one forward + backward (parameter gradients only, as training_helpers.py:141-144 produces)
 of the layer over one batch of synthetic features that are already resident in HBM; for N > 1 the
@@ -86,6 +87,7 @@ class SSSWorkload:
 
     def make_layer(self, device):
         from structurednets_b200.layers.sss_layer import SSSLayer
+        np.random.seed(5000)      # the bias is Glorot-initialised from numpy's global RNG: every run builds the same layer
         layer = SSSLayer(self.input_dim, self.output_dim, 0.105, nb_states=self.nb_states, initial_system_approx=self.system())
         assert layer.statespace_dim == self.statespace_dim
         return layer.to(device)
@@ -216,6 +218,7 @@ class PSMWorkload(_DenseInputsMixin):
 
     def make_layer(self, device):
         from structurednets_b200.layers.psm_layer import PSMLayer
+        np.random.seed(3000)      # Glorot bias, as in SSSWorkload.make_layer
         return PSMLayer(self.input_dim, self.output_dim, sparse_matrices=self.factors()).to(device)
 
     def ref_step_fn(self, batch, device="cpu"):
@@ -270,6 +273,7 @@ class HMatWorkload(_DenseInputsMixin):
 
     def make_layer(self, device):
         from structurednets_b200.layers.hmat_layer import HMatLayer
+        np.random.seed(4000)      # Glorot bias, as in SSSWorkload.make_layer
         return HMatLayer(self.input_dim, self.output_dim, 0.2, initial_hmatrix=self.hmatrix()).to(device)
 
     def ref_step_fn(self, batch, device="cpu"):
@@ -429,6 +433,41 @@ def cpu_model():
     return "unknown"
 
 
+DUMP_BYTES = 64 * 2 ** 20
+
+
+def step_outputs(runner, y):
+    """What a caller of the timed step receives: the layer output and the parameter gradients (`grad_flat` is the buffer every dense
+    float32 parameter's .grad is a view of, in named_parameters() order; the other parameters' gradients are listed by name)."""
+    out = {"y": y}
+    if runner.has_flat:
+        out["grad_flat"] = runner.layer.flat_grad()
+    loose = set(map(id, runner.loose))
+    for name, p in runner.layer.named_parameters():
+        if id(p) in loose and p.grad is not None:
+            out["grad." + name] = p.grad
+    return out
+
+
+def dump_outputs(path, arrays):
+    """Writes every tensor of `arrays` to path/<name>.npy, float64 as float64 and everything else as float32, DUMP_BYTES in all.
+    An array larger than its equal share keeps a sample of its rows (of its entries if one row is too large) drawn from a fixed
+    seed, so two runs with the same arguments store the same elements."""
+    os.makedirs(path, exist_ok=True)
+    share = (DUMP_BYTES - 4096 * len(arrays)) // len(arrays)      # 4 KB per file left for the .npy header
+    for name, t in arrays.items():
+        t = t.detach()
+        t = t.to_dense() if t.is_sparse else t
+        t = t if t.dtype == torch.float64 else t.float()
+        if t.dim() == 0 or t[0].numel() * t.element_size() > share:
+            t = t.reshape(-1)
+        keep = share // (t[0].numel() * t.element_size())
+        if t.shape[0] > keep:
+            idx = np.sort(np.random.default_rng(0).choice(t.shape[0], keep, replace=False))
+            t = t.index_select(0, torch.from_numpy(idx).to(t.device))
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
+
+
 def time_reference_steps(wl, steps, warmup, budget_s=25.0, device="cpu", batch=None):
     """The reference's own ops (oracle port) for this workload on `device`: host cores (cpu_baseline, --impl reference) or the same
     B200 (gpu_aten_baseline: what the reference's use_gpu=True runs)."""
@@ -466,7 +505,7 @@ def run_reference(args, wl):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    base, med, n = time_reference_steps(wl, steps=max(args.steps, 2), warmup=max(args.warmup, 1), budget_s=120.0)
+    base, med, n = time_reference_steps(wl, steps=args.steps, warmup=max(args.warmup, 1), budget_s=float("inf"))
     cfg = wl.describe()
     cfg["sample_batch"] = wl.cpu_sample_batch
     line = dict(metric="structured-layer fwd+bwd samples/sec", value=base["value"], unit="samples/s", n_gpus=args.gpus, steps=n,
@@ -535,9 +574,27 @@ def _ev():
     return torch.cuda.Event(enable_timing=True)
 
 
-def measure(runner, steps, warmup, peaks, local_rank, barrier, use_graph=True, sustained_s=0.0):
+def _last_output(y, last):
+    """The step's output if it is the last one, else None (freed before the next step allocates its own, as when it is dropped).
+    Detached: a live autograd graph of an earlier step makes a later CUDA-graph capture fail (its backward would wait on
+    uncaptured work)."""
+    return y.detach() if last else None
+
+
+def _capture(runner, n):
+    """A CUDA graph of steps 0 .. n-1 and the output of its last step (kept alive, so replays refresh it)."""
+    graph = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(graph):
+        for k in range(n):
+            y = _last_output(runner.step(k), k == n - 1)
+    return graph, y
+
+
+def measure(runner, steps, warmup, peaks, local_rank, barrier, use_graph=True, sustained_s=0.0, last_step=None):
     """Eager pass (per-kernel CUDA-event pairs recorded by the library around each of its launches) + CUDA-graph pass (the number
-    reported).  Returns a dict; all times in ms, device-timed with CUDA events on the launching stream."""
+    reported), each of exactly `steps` steps.  Returns a dict; all times in ms, device-timed with CUDA events on the launching stream.
+    `last_step(y)`, if given, is called with the output of the reported pass's last step while the layer's gradients are still
+    that step's."""
     from structurednets_b200 import _lib
     wl, stream = runner.wl, runner.stream
     _lib.lib().sn_timing_enable(1)
@@ -552,7 +609,7 @@ def measure(runner, steps, warmup, peaks, local_rank, barrier, use_graph=True, s
         barrier()
         t_begin.record(stream)
         for i in range(steps):
-            runner.step(i, recs[i])
+            y = _last_output(runner.step(i, recs[i]), i == steps - 1)
         t_end.record(stream)
         barrier()
     launches = _lib.launch_count()
@@ -572,28 +629,39 @@ def measure(runner, steps, warmup, peaks, local_rank, barrier, use_graph=True, s
                 runner.step(0)
             torch.cuda.current_stream().wait_stream(side)
             torch.cuda.synchronize()
-            graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(graph):
-                for k in range(runner.n_sets):
-                    runner.step(k)
+            graph, y = _capture(runner, runner.n_sets)
+            # steps that are not a multiple of the input sets end with a graph of the first (steps mod n_sets) sets
+            reps, rest = divmod(steps, runner.n_sets)
+            tail = None
+            if rest:
+                tail, y = _capture(runner, rest)
             for _ in range(3):
                 graph.replay()
+                if tail is not None:
+                    tail.replay()
             torch.cuda.synchronize()
-            reps = max(1, -(-steps // runner.n_sets))
             g0, g1 = _ev(), _ev()
             with ClockSampler(local_rank) as clocks:
                 barrier()
                 g0.record()
                 for _ in range(reps):
                     graph.replay()
+                if tail is not None:
+                    tail.replay()
                 g1.record()
                 barrier()
-            elapsed_ms, timed_steps = g0.elapsed_time(g1), reps * runner.n_sets
+            elapsed_ms = g0.elapsed_time(g1)
             graph_note = "CUDA graph of %d step(s) (one per input set), replayed %d times" % (runner.n_sets, reps)
+            if tail is not None:
+                graph_note += ", then a graph of the first %d" % rest
         except Exception as e:   # a layer whose step cannot be captured (host synchronisation inside) keeps the eager number
             torch.cuda.synchronize()
             graph = None
             graph_note = "eager launches (graph capture failed: %s)" % str(e).splitlines()[0][:120]
+            if last_step is not None:   # the warm-up step above overwrote the gradients: the eager pass's last step once more
+                y = runner.step(steps - 1).detach()
+    if last_step is not None:
+        last_step(y)
     out.update(elapsed_ms=elapsed_ms, timed_steps=timed_steps, launch_mode=graph_note, clocks=clocks.summary())
     if sustained_s > 0 and graph is not None:
         ms = elapsed_ms / timed_steps * runner.n_sets
@@ -779,8 +847,11 @@ def run_ours(args, wl):
         dp_ok, dp_detail = dp_check(runner, n_gpus, rank, device)
 
     grad_transport = runner.grad_sync.transport if (n_gpus > 1 and runner.grad_sync is not None and hasattr(runner.grad_sync, "transport")) else None
+    last_step = None
+    if args.dump_outputs and rank == 0:
+        last_step = lambda y: dump_outputs(args.dump_outputs, step_outputs(runner, y))
     m = measure(runner, args.steps, args.warmup, peaks, local_rank, barrier, use_graph=not args.no_graph,
-                sustained_s=2.5 if (n_gpus == 1 and not args.quick) else 0.0)
+                sustained_s=2.5 if (n_gpus == 1 and not args.quick) else 0.0, last_step=last_step)
     elapsed_ms = m["elapsed_ms"]
     if n_gpus > 1:
         t = torch.tensor([elapsed_ms], device=device)
@@ -879,7 +950,14 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="time eager launches instead of CUDA-graph replays")
     ap.add_argument("--quick", action="store_true", help="headline workload only: no sustained run, no secondary workloads (profiling)")
     ap.add_argument("--global-batch", type=int, default=None, help="profiling only: override the workload's global batch")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's output and parameter gradients to DIR/<name>.npy (rank 0's "
+                         "shard; 64 MB in all, larger arrays as a fixed sample of their rows); inputs are seeded, so runs compare")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or getattr(WORKLOADS[args.workload], "host_features", False)):
+        ap.error("--dump-outputs is for --impl ours on a workload with resident inputs")
     wl = WORKLOADS[args.workload]()
     if args.global_batch:
         wl.global_batch = args.global_batch

@@ -15,11 +15,12 @@ import os
 import sys
 import types
 
-REFERENCE_SRC = "/root/reference/src"
+# a checkout of MatthiasKi/structurednets, given by the same variable as in oracle/run_c.py
+REFERENCE_SRC = os.path.join(os.environ["SNB200_REFERENCE"], "src") if os.environ.get("SNB200_REFERENCE") else None
 
 
 def reference_available() -> bool:
-    return os.path.isdir(os.path.join(REFERENCE_SRC, "structurednets"))
+    return REFERENCE_SRC is not None and os.path.isdir(os.path.join(REFERENCE_SRC, "structurednets"))
 
 
 def _stub(name, **attrs):

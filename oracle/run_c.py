@@ -15,7 +15,9 @@ import tempfile
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_SRC = os.environ.get("SNB200_REFERENCE", "/root/reference") + "/src/structurednets/speed_comparison/run.c"
+# SNB200_REFERENCE: a checkout of MatthiasKi/structurednets
+REF_SRC = (os.path.join(os.environ["SNB200_REFERENCE"], "src/structurednets/speed_comparison/run.c")
+           if os.environ.get("SNB200_REFERENCE") else None)
 REF_BIN = os.path.join(HERE, "_ref", "run")
 
 
@@ -23,7 +25,7 @@ def build_ref(force: bool = False):
     """gcc on the reference's run.c (its own header says ``gcc -o run run.c``, run.c:10).  Returns the binary path or None."""
     if os.path.exists(REF_BIN) and not force:
         return REF_BIN
-    if not os.path.exists(REF_SRC):
+    if REF_SRC is None or not os.path.exists(REF_SRC):
         return None
     os.makedirs(os.path.dirname(REF_BIN), exist_ok=True)
     subprocess.run(["gcc", "-O1", "-o", REF_BIN, REF_SRC, "-lm"], check=True, capture_output=True)

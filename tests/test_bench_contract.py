@@ -1,9 +1,12 @@
-"""bench.py's reference arm runs without a GPU: its JSON line must carry the keys the driver reads (the GPU arm's line is produced
-on the B200 at round end; its extra keys are checked here only by name in the source)."""
+"""bench.py's reference arm runs without a GPU and its JSON line must carry the result keys; the GPU arm's extra keys are checked
+here by name in the source.  On a GPU: the timed step count and the output dump."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -28,3 +31,27 @@ def test_gpu_arm_emits_the_contract_keys():
     for key in ("roofline", "cpu_baseline", "e2e", "gpu_launches", "clocks", "h2d_bytes_per_step", "d2h_bytes_per_step", "traffic",
                 "ms_per_step", "higher_is_better", "scaling", "vs_baseline", "sm_max_mhz", "reasons"):
         assert key in src, key
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_timed_step(tmp_path, built_lib):
+    """At batch 4096 the SSS workload rotates four input sets; --steps 3 must time exactly three steps, and --dump-outputs must hold
+    the output and parameter gradients of the third one, as one eager step on the same seeded layer and inputs computes them."""
+    import torch
+    import bench
+    r = subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), "--steps", "3", "--warmup", "1", "--quick", "--no-cpu-baseline",
+                        "--global-batch", "4096", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900, cwd=REPO)
+    assert r.returncode == 0, r.stderr[-2000:]
+    d = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+    assert d["steps"] == 3
+    assert d["config"]["launch_mode"].startswith("CUDA graph"), d["config"]["launch_mode"]     # the dump must not cost the capture
+    assert sorted(os.listdir(tmp_path)) == ["grad_flat.npy", "y.npy"]
+    wl = bench.SSSWorkload()
+    runner = bench.StepRunner(wl, torch.device("cuda"), 4096, seed=5000)
+    assert runner.n_sets == 4
+    y = runner.step(2)
+    for name, ref in (("y", y), ("grad_flat", runner.layer.flat_grad())):
+        got = np.load(tmp_path / (name + ".npy"))
+        ref = ref.detach().cpu().numpy()
+        assert got.dtype == np.float32 and got.shape == ref.shape, name
+        assert np.abs(got - ref).max() <= 1e-5 * np.abs(ref).max(), name

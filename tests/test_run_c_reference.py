@@ -15,7 +15,8 @@ CASES = [dict(i=76, o=14, n=7, d=5, ragged=True), dict(i=128, o=24, n=12, d=16, 
 
 def _binary_or_skip():
     if run_c.build_ref() is None:
-        pytest.skip("oracle/_ref/run is not built (needs the reference source in the build container)")
+        pytest.skip("oracle/_ref/run is not built: it is compiled from the reference project's speed_comparison/run.c, which is not "
+                    "part of this repository (set SNB200_REFERENCE to a checkout of MatthiasKi/structurednets)")
 
 
 def _layer(case, seed=3):

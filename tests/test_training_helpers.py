@@ -182,7 +182,8 @@ def test_live_reference_train_when_the_reference_tree_is_present():
     """Same comparison against the imported reference itself (build container only; skipped on the GPU box)."""
     from oracle.ref_import import load_reference, reference_available
     if not reference_available():
-        pytest.skip("/root/reference is not present")
+        pytest.skip("the reference project is not part of this repository (set SNB200_REFERENCE to a checkout of "
+                    "MatthiasKi/structurednets); tests/golden/train_linear.npz holds its results")
     load_reference()
     from structurednets import training_helpers as RTH
     from tests.golden.make_golden import train_case
