@@ -272,6 +272,35 @@ int sn_dense_weight_grad(const float* x, int64_t ldx, const float* grad_y, int64
                          float* grad_bias, int64_t B, sn_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
+ * bf16 features on the dense-product layers (PSM dense path, H-matrix dense-block path, LDR, TL), csrc/dense_bf16.cu:
+ * W is still built in fp32 from the layer's parameters; these entries run the batch GEMMs on bf16 tensor cores (fp32
+ * accumulation in TMEM).  x, grad_y, y, grad_x and the W copies are bf16 ("void*"), dW and the gradients fp32.  Every bf16
+ * operand needs a 16-byte aligned base and a row pitch that is a multiple of 8 elements.
+ *   sn_dense_cast_bf16: Mb = bf16(M) [rows][ldmb] and / or Mtb = bf16(M)^T [cols][ldmtb] (either nullable) in one pass over
+ *     the fp32 M [rows][cols]; pad columns are zeroed.
+ *   sn_dense_apply_bf16: y = x W^T + bias (bf16 store); Wb = W bf16 [n_out][ldwb].
+ *   sn_dense_weight_grad_bf16: dW [n_out][lddw] += grad_y^T x in fp32 (split-K over the batch, fp32 reductions),
+ *     grad_bias += column sums of grad_y.
+ *   sn_dense_input_grad_bf16: grad_x = grad_y W (bf16 store); Wtb = W^T bf16 [n_in][ldwtb].
+ * ------------------------------------------------------------------------------------------ */
+int sn_dense_cast_bf16(const float* M, int rows, int cols, void* Mb, int64_t ldmb, void* Mtb, int64_t ldmtb, sn_stream_t stream);
+int sn_dense_apply_bf16(const void* Wb, int64_t ldwb, int n_out, int n_in, const void* x, int64_t ldx, void* y, int64_t ldy,
+                        const float* bias, int64_t B, sn_stream_t stream);
+int sn_dense_weight_grad_bf16(const void* x, int64_t ldx, const void* grad_y, int64_t ldgy, float* dW, int64_t lddw, int n_out,
+                              int n_in, float* grad_bias, int64_t B, sn_stream_t stream);
+int sn_dense_input_grad_bf16(const void* Wtb, int64_t ldwtb, int n_out, int n_in, const void* grad_y, int64_t ldgy, void* grad_x,
+                             int64_t ldgx, int64_t B, sn_stream_t stream);
+/* PSM dense-product path with bf16 features: the prefix products and the projection of sn_psm_dense_forward / _backward, the
+ * batch GEMMs above.  wb = W bf16 [out_dim][ldwb] and wtb = W^T bf16 [in_dim][ldwtb] (nullable) are written by the forward;
+ * grad_x = sn_dense_input_grad_bf16(wtb, ...). */
+int sn_psm_dense_forward_bf16(const sn_psm_dense_factor* factors_host, int nf, const void* x, int64_t ldx, void* y, int64_t ldy,
+                              const float* bias, float* prefix, void* wb, int64_t ldwb, void* wtb, int64_t ldwtb, int64_t B,
+                              int in_dim, int out_dim, sn_stream_t stream);
+int sn_psm_dense_backward_bf16(const sn_psm_dense_factor* factors_host, int nf, const void* x, int64_t ldx, const void* grad_y,
+                               int64_t ldgy, const float* prefix, float* work, float* grad_bias, int64_t B, int in_dim, int out_dim,
+                               sn_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
  * Toeplitz-like layer -- replaces the weight construction of TLLayer.forward (layers/tl_layer.py:11-18,59) and
  * its backward.  G (n x r), H (r x n) float32; K1 (n x rn) and K2 (rn x n) are scratch kept for the backward.
  * ------------------------------------------------------------------------------------------ */

@@ -137,6 +137,18 @@ def _declare(lib):
     lib.sn_tl_build_weight.argtypes = [i32, i32, vp, vp, vp, vp, vp, vp]
     lib.sn_tl_backward.restype = c_int
     lib.sn_tl_backward.argtypes = [i32, i32, vp, vp, vp, vp, vp, vp, vp, vp]
+    lib.sn_dense_cast_bf16.restype = c_int
+    lib.sn_dense_cast_bf16.argtypes = [vp, i32, i32, vp, i64, vp, i64, vp]
+    lib.sn_dense_apply_bf16.restype = c_int
+    lib.sn_dense_apply_bf16.argtypes = [vp, i64, i32, i32, vp, i64, vp, i64, vp, i64, vp]
+    lib.sn_dense_weight_grad_bf16.restype = c_int
+    lib.sn_dense_weight_grad_bf16.argtypes = [vp, i64, vp, i64, vp, i64, i32, i32, vp, i64, vp]
+    lib.sn_dense_input_grad_bf16.restype = c_int
+    lib.sn_dense_input_grad_bf16.argtypes = [vp, i64, i32, i32, vp, i64, vp, i64, i64, vp]
+    lib.sn_psm_dense_forward_bf16.restype = c_int
+    lib.sn_psm_dense_forward_bf16.argtypes = [PD, i32, vp, i64, vp, i64, vp, vp, vp, i64, vp, i64, i64, i32, i32, vp]
+    lib.sn_psm_dense_backward_bf16.restype = c_int
+    lib.sn_psm_dense_backward_bf16.argtypes = [PD, i32, vp, i64, vp, i64, vp, vp, vp, i64, i32, i32, vp]
     lib.sn_lr_tc_cast_params.restype = c_int
     lib.sn_lr_tc_cast_params.argtypes = [vp, vp, vp, vp, i64, vp, i32, i32, i32, vp]
     lib.sn_lr_tc_forward.restype = c_int

@@ -11,6 +11,7 @@
 // The batch-reduction GEMMs run on bf16 transposes made by a tiled transpose kernel (ranks that are not a multiple of 64);
 // otherwise the activations are consumed in their natural [sample][feature] layout through MN-major UMMA descriptors.
 #include <stdlib.h>
+#include "bf16_ops.cuh"
 #include "gemm_tc.cuh"
 
 namespace {
@@ -31,48 +32,6 @@ __global__ void lr_cast_params_kernel(const float* __restrict__ left, const floa
             Rb[e - nl] = __float2bfloat16(right[e - nl]);
         }
     }
-}
-
-// dst[c][r] = src[r][c]  (bf16, 32x32 tiles through shared memory)
-__global__ void transpose_bf16_kernel(const bf16* __restrict__ src, long lds, bf16* __restrict__ dst, long ldd, long rows, int cols) {
-    __shared__ bf16 tile[32][33];
-    const long r0 = (long)blockIdx.y * 32;
-    const int c0 = blockIdx.x * 32;
-    for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-        const long r = r0 + i;
-        const int c = c0 + threadIdx.x;
-        tile[i][threadIdx.x] = (r < rows && c < cols) ? src[r * lds + c] : __float2bfloat16(0.f);
-    }
-    __syncthreads();
-    for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-        const int c = c0 + i;
-        const long r = r0 + threadIdx.x;
-        if (c < cols && r < rows) dst[(size_t)c * ldd + r] = tile[threadIdx.x][i];
-    }
-}
-
-// out[c] += sum_r M[r][c]: a thread owns a pair of columns (one 4-byte load per row, coalesced along the row), 64-row slabs
-__global__ void colsum_bf16_kernel(const bf16* __restrict__ M, long ld, long rows, int cols, float* __restrict__ out) {
-    const int c = 2 * (blockIdx.x * blockDim.x + threadIdx.x);
-    if (c >= cols) return;
-    const long r0 = (long)blockIdx.y * 64;
-    const long r1 = r0 + 64 < rows ? r0 + 64 : rows;
-    float s0 = 0.f, s1 = 0.f;
-    if (c + 1 < cols && (ld & 1) == 0 && ((reinterpret_cast<uintptr_t>(M) & 3) == 0)) {
-#pragma unroll 8
-        for (long r = r0; r < r1; ++r) {
-            const __nv_bfloat162 v = *reinterpret_cast<const __nv_bfloat162*>(M + r * ld + c);
-            s0 += __bfloat162float(v.x);
-            s1 += __bfloat162float(v.y);
-        }
-    } else {
-        for (long r = r0; r < r1; ++r) {
-            s0 += __bfloat162float(M[r * ld + c]);
-            if (c + 1 < cols) s1 += __bfloat162float(M[r * ld + c + 1]);
-        }
-    }
-    atomicAdd(out + c, s0);
-    if (c + 1 < cols) atomicAdd(out + c + 1, s1);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -270,22 +229,9 @@ lr_tc_fwd_fused_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_c
     }
 }
 
-int transpose_bf16(const bf16* src, long lds, bf16* dst, long ldd, long rows, int cols, cudaStream_t st) {
-    dim3 grid(snb::ceil_div(cols, 32), (unsigned)((rows + 31) / 32)), block(32, 8);
-    SN_LAUNCH("transpose_bf16_kernel", st, transpose_bf16_kernel<<<grid, block, 0, st>>>(src, lds, dst, ldd, rows, cols));
-    return 0;
-}
-
 // (SideStream / side_stream(): common.cuh)  The bias gradient and dL run next to gh -> dR on a second stream.
 using snb::SideStream;
 using snb::side_stream;
-
-inline int split_for(int tiles, long K) {
-    int want = snb::ceil_div(148, tiles > 0 ? tiles : 1);
-    long maxs = (K + 511) / 512;   // at least 512 of K per slice
-    if (want > maxs) want = (int)maxs;
-    return want < 1 ? 1 : want;
-}
 
 }  // namespace
 

@@ -13,6 +13,7 @@
 // from the parameter's own COO array into that order once per call (psm_pack_vals_kernel); the backward
 // accumulates dS in the same packed order with coalesced reductions and scatters it back once.
 #include "common.cuh"
+#include "bf16_ops.cuh"
 #include "util.cuh"
 #include "gemm_f32.cuh"
 
@@ -384,6 +385,51 @@ int check_dense_chain(const sn_psm_dense_factor* f, int nf, int in_dim, int out_
     return 0;
 }
 
+// prefix: L_1^T | L_2^T | ... | L_n^T = W^T ([cols_{k-1}][out_dim] each); returns W^T (the last block) in *wt
+int build_prefix(const sn_psm_dense_factor* f, int nf, float* prefix, int out_dim, const float** wt, cudaStream_t st) {
+    float* cur = prefix;
+    const float* prev = nullptr;
+    for (int k = 0; k < nf; ++k) {
+        // L_{k+1}^T = S_k^T L_k^T: the rows of S_k^T are the columns of S_k (csc)
+        // (the pipelined row kernel of the backward, without its dot products, is slower here: 45 vs 35 us per factor at C3)
+        SN_LAUNCH("psm_rowcomb_kernel", st, psm_rowcomb_kernel<<<f[k].cols, 256, 0, st>>>(f[k].csc_ptr, f[k].csc_idx, f[k].csc_src, f[k].vals, prev, cur, out_dim));
+        prev = cur;
+        cur += (size_t)f[k].cols * out_dim;
+    }
+    *wt = prev;
+    return 0;
+}
+
+// Projection of the dense gradient onto every factor's pattern.  work starts with H_{n-1}^T = G^T = x^T grad_y [in_dim][out_dim];
+// the suffix recursion writes H_{n-2}^T [rows_{n-1}][out_dim], ... behind it.
+int project_dense_grad(const sn_psm_dense_factor* f, int nf, const float* prefix, float* work, int out_dim, cudaStream_t st) {
+    float* Ht = work;
+    // prefix offsets: L_k^T for k >= 1 starts after the first k - 1 blocks
+    size_t off[PSM_MAX_FACTORS + 1];
+    off[0] = 0;
+    for (int k = 0; k < nf; ++k) off[k + 1] = off[k] + (size_t)f[k].cols * out_dim;
+    for (int k = nf - 1; k >= 0; --k) {
+        const float* Lt = k == 0 ? nullptr : prefix + off[k - 1];
+        if (k > 0 && out_dim <= 4 * 32 * PBR_NI) {
+            // gradient of the factor's non-zeros and the next adjoint H_{k-1}^T = S_k H_k^T [rows_k][out_dim] in one pass over H_k^T
+            float* Hn = Ht + (size_t)f[k].cols * out_dim;
+            SN_LAUNCH("psm_bwd_row_kernel", st, psm_bwd_row_kernel<true><<<f[k].rows, PBR_WARPS * 32, 0, st>>>(f[k].csr_ptr, f[k].csr_idx, f[k].csr_src, f[k].vals, Lt, Ht,
+                                                                                                       f[k].grad_vals, Hn, out_dim));
+            Ht = Hn;
+            continue;
+        }
+        if (f[k].nnz > 0 && f[k].grad_vals != nullptr)
+            SN_LAUNCH("psm_masked_dot_kernel", st, psm_masked_dot_kernel<<<(unsigned)(((size_t)f[k].nnz * (Lt == nullptr ? 1 : 32) + 255) / 256), 256, 0, st>>>(
+                f[k].coo_row, f[k].coo_col, f[k].nnz, Lt, Ht, f[k].grad_vals, out_dim));
+        if (k > 0) {
+            float* Hn = Ht + (size_t)f[k].cols * out_dim;   // H_{k-1}^T = S_k H_k^T: [rows_k][out_dim]
+            SN_LAUNCH("psm_rowcomb_kernel", st, psm_rowcomb_kernel<<<f[k].rows, 256, 0, st>>>(f[k].csr_ptr, f[k].csr_idx, f[k].csr_src, f[k].vals, Ht, Hn, out_dim));
+            Ht = Hn;
+        }
+    }
+    return 0;
+}
+
 }  // namespace
 
 extern "C" {
@@ -462,17 +508,10 @@ int sn_psm_dense_forward(const sn_psm_dense_factor* f, int nf, const float* x, i
     SN_CHECK_ARG(x && y && prefix, "psm_dense_forward: NULL buffer");
     if (B <= 0) return 0;
     cudaStream_t st = snb::as_stream(stream);
-    float* cur = prefix;
-    const float* prev = nullptr;
-    for (int k = 0; k < nf; ++k) {
-        // L_{k+1}^T = S_k^T L_k^T: the rows of S_k^T are the columns of S_k (csc)
-        // (the pipelined row kernel of the backward, without its dot products, is slower here: 45 vs 35 us per factor at C3)
-        SN_LAUNCH("psm_rowcomb_kernel", st, psm_rowcomb_kernel<<<f[k].cols, 256, 0, st>>>(f[k].csc_ptr, f[k].csc_idx, f[k].csc_src, f[k].vals, prev, cur, out_dim));
-        prev = cur;
-        cur += (size_t)f[k].cols * out_dim;
-    }
+    const float* wt = nullptr;
+    if (int rc = build_prefix(f, nf, prefix, out_dim, &wt, st)) return rc;
     // y = x W^T^T + b: W^T is stored [in_dim][out_dim]
-    return snb::gemm_f32(false, false, (int)B, out_dim, in_dim, 1.f, x, ldx, prev, out_dim, 0.f, y, ldy, bias, st);
+    return snb::gemm_f32(false, false, (int)B, out_dim, in_dim, 1.f, x, ldx, wt, out_dim, 0.f, y, ldy, bias, st);
 }
 /* grad_x = grad_y W from the multiplied-out product the forward left in `prefix` (W^T = its last block, [in_dim][out_dim]) */
 int sn_psm_dense_input_grad(const sn_psm_dense_factor* f, int nf, const float* prefix, const float* grad_y, int64_t ldgy, float* grad_x,
@@ -497,30 +536,36 @@ int sn_psm_dense_backward(const sn_psm_dense_factor* f, int nf, const float* x, 
     float* Ht = work;
     SN_CHECK_CUDA(cudaMemsetAsync(Ht, 0, (size_t)in_dim * out_dim * sizeof(float), st));
     if (int rc = snb::gemm_f32(true, false, in_dim, out_dim, (int)B, 1.f, x, ldx, grad_y, ldgy, 1.f, Ht, out_dim, nullptr, st, true)) return rc;
-    // prefix offsets: L_k^T for k >= 1 starts after the first k - 1 blocks
-    size_t off[PSM_MAX_FACTORS + 1];
-    off[0] = 0;
-    for (int k = 0; k < nf; ++k) off[k + 1] = off[k] + (size_t)f[k].cols * out_dim;
-    for (int k = nf - 1; k >= 0; --k) {
-        const float* Lt = k == 0 ? nullptr : prefix + off[k - 1];
-        if (k > 0 && out_dim <= 4 * 32 * PBR_NI) {
-            // gradient of the factor's non-zeros and the next adjoint H_{k-1}^T = S_k H_k^T [rows_k][out_dim] in one pass over H_k^T
-            float* Hn = Ht + (size_t)f[k].cols * out_dim;
-            SN_LAUNCH("psm_bwd_row_kernel", st, psm_bwd_row_kernel<true><<<f[k].rows, PBR_WARPS * 32, 0, st>>>(f[k].csr_ptr, f[k].csr_idx, f[k].csr_src, f[k].vals, Lt, Ht,
-                                                                                                       f[k].grad_vals, Hn, out_dim));
-            Ht = Hn;
-            continue;
-        }
-        if (f[k].nnz > 0 && f[k].grad_vals != nullptr)
-            SN_LAUNCH("psm_masked_dot_kernel", st, psm_masked_dot_kernel<<<(unsigned)(((size_t)f[k].nnz * (Lt == nullptr ? 1 : 32) + 255) / 256), 256, 0, st>>>(
-                f[k].coo_row, f[k].coo_col, f[k].nnz, Lt, Ht, f[k].grad_vals, out_dim));
-        if (k > 0) {
-            float* Hn = Ht + (size_t)f[k].cols * out_dim;   // H_{k-1}^T = S_k H_k^T: [rows_k][out_dim]
-            SN_LAUNCH("psm_rowcomb_kernel", st, psm_rowcomb_kernel<<<f[k].rows, 256, 0, st>>>(f[k].csr_ptr, f[k].csr_idx, f[k].csr_src, f[k].vals, Ht, Hn, out_dim));
-            Ht = Hn;
-        }
-    }
-    return 0;
+    return project_dense_grad(f, nf, prefix, Ht, out_dim, st);
+}
+
+/* bf16 features: the same prefix products and projection as above, the batch GEMMs on the bf16 tensor cores of csrc/dense_bf16.cu.
+   wb: W bf16 [out_dim][ldwb], written; wtb: W^T bf16 [in_dim][ldwtb], written when not null (sn_dense_input_grad_bf16 reads it). */
+int sn_psm_dense_forward_bf16(const sn_psm_dense_factor* f, int nf, const void* x, int64_t ldx, void* y, int64_t ldy, const float* bias,
+                              float* prefix, void* wb, int64_t ldwb, void* wtb, int64_t ldwtb, int64_t B, int in_dim, int out_dim,
+                              sn_stream_t stream) {
+    if (int rc = check_dense_chain(f, nf, in_dim, out_dim)) return rc;
+    SN_CHECK_ARG(x && y && prefix && wb, "psm_dense_forward_bf16: NULL buffer");
+    if (B <= 0) return 0;
+    const float* wt = nullptr;
+    if (int rc = build_prefix(f, nf, prefix, out_dim, &wt, snb::as_stream(stream))) return rc;
+    // the last prefix block is W^T [in_dim][out_dim]: its copy is W^T, its transpose W
+    if (int rc = sn_dense_cast_bf16(wt, in_dim, out_dim, wtb, ldwtb, wb, ldwb, stream)) return rc;
+    return sn_dense_apply_bf16(wb, ldwb, out_dim, in_dim, x, ldx, y, ldy, bias, B, stream);
+}
+int sn_psm_dense_backward_bf16(const sn_psm_dense_factor* f, int nf, const void* x, int64_t ldx, const void* grad_y, int64_t ldgy,
+                               const float* prefix, float* work, float* grad_bias, int64_t B, int in_dim, int out_dim, sn_stream_t stream) {
+    if (int rc = check_dense_chain(f, nf, in_dim, out_dim)) return rc;
+    SN_CHECK_ARG(x && grad_y && prefix && work, "psm_dense_backward_bf16: NULL buffer");
+    if (B <= 0) return 0;
+    cudaStream_t st = snb::as_stream(stream);
+    if (grad_bias)
+        if (int rc = colsum_bf16((const __nv_bfloat16*)grad_y, ldgy, B, out_dim, grad_bias, st)) return rc;
+    float* Ht = work;
+    SN_CHECK_CUDA(cudaMemsetAsync(Ht, 0, (size_t)in_dim * out_dim * sizeof(float), st));
+    // H_{n-1}^T = x^T grad_y [in_dim][out_dim]: the weight-gradient GEMM with the roles of the features and grad_y swapped
+    if (int rc = sn_dense_weight_grad_bf16(grad_y, ldgy, x, ldx, Ht, out_dim, in_dim, out_dim, nullptr, B, stream)) return rc;
+    return project_dense_grad(f, nf, prefix, Ht, out_dim, st);
 }
 
 }  // extern "C"

@@ -11,6 +11,7 @@ import torch
 import torch.nn as nn
 
 from structurednets_b200 import _lib
+from structurednets_b200.layers import dense_bf16 as D
 from structurednets_b200.hmatrix.hmatrix import BlockClusterTree, HMatrix, HMatrixComponent, TreeElement, approximate_hmatrix
 from structurednets_b200.layers.flat_params import FlatParamsMixin
 from structurednets_b200.layers.layer_helpers import get_random_glorot_uniform_matrix
@@ -95,6 +96,44 @@ class _HMatDenseFunction(torch.autograd.Function):
         slabs = layer._slab_table(U.device)
         _lib.check(L.sn_hmat_project_grad(_lib.ptr(table), layer._nleaves, _lib.ptr(slabs), slabs.numel() // 2, _lib.ptr(layer.flat_parameters()),
                                           _lib.ptr(dW), layer.output_dim, layer.input_dim, _lib.ptr(g), _lib.stream_ptr()), "sn_hmat_project_grad")
+        return grad_x, None, None
+
+
+class _HMatDenseBF16Function(torch.autograd.Function):
+    """bfloat16 features on the dense-block path: the same float32 W (sn_hmat_build_dense) and projection (sn_hmat_project_grad),
+    the batch GEMMs on bf16 tensor cores (layers/dense_bf16.py).  Like the float32 path, the projection reads the layer's current
+    parameters: forward -> backward without a parameter update in between."""
+
+    @staticmethod
+    def forward(ctx, U, anchor, layer):
+        L = _lib.lib()
+        table = layer._leaf_table(U.device)
+        W = layer._dense_buffer("_dev_W", U.device)
+        slabs = layer._slab_table(U.device)
+        _lib.check(L.sn_hmat_build_dense(_lib.ptr(table), layer._nleaves, layer._max_leaf_rows, _lib.ptr(slabs), slabs.numel() // 2,
+                                         _lib.ptr(layer.flat_parameters()), _lib.ptr(W), layer.output_dim, layer.input_dim, _lib.stream_ptr()),
+                   "sn_hmat_build_dense")
+        x = D.staged(U)
+        y, Wtb = D.forward(layer, W, x, layer.bias if layer.use_bias else None, keep_wt=ctx.needs_input_grad[0])
+        ctx.layer = layer
+        ctx.save_for_backward(x, table, Wtb)
+        return y
+
+    @staticmethod
+    def backward(ctx, grad_y):
+        layer = ctx.layer
+        x, table, Wtb = ctx.saved_tensors
+        gy = D.staged(grad_y)
+        grad_x = D.input_grad(Wtb, gy) if ctx.needs_input_grad[0] else None
+        g = layer._prepare_grad_accumulation()
+        gb = g[:layer.output_dim] if (layer.use_bias and layer.bias.requires_grad) else None
+        dW = layer._dense_buffer("_dev_dW", x.device)
+        dW.zero_()
+        D.weight_grad(x, gy, dW, gb)
+        slabs = layer._slab_table(x.device)
+        _lib.check(_lib.lib().sn_hmat_project_grad(_lib.ptr(table), layer._nleaves, _lib.ptr(slabs), slabs.numel() // 2,
+                                                   _lib.ptr(layer.flat_parameters()), _lib.ptr(dW), layer.output_dim, layer.input_dim, _lib.ptr(g),
+                                                   _lib.stream_ptr()), "sn_hmat_project_grad")
         return grad_x, None, None
 
 
@@ -222,16 +261,19 @@ class HMatLayer(FlatParamsMixin, StructuredLayer):
         self._require_cuda(U, "HMatLayer.forward")
         assert U.dim() == 2 and U.shape[1] == self.input_dim, "HMatLayer expects a (batch, input_dim) input"
         self._ensure_flat()
-        if U.dtype != torch.float32:
-            U = U.float()
-        if U.stride(1) != 1:
-            U = U.contiguous()
+        if U.dtype == torch.bfloat16 and self._use_dense_path():   # bf16 output, float32 parameters and gradients
+            fn = _HMatDenseBF16Function
+        else:
+            fn = _HMatDenseFunction if self._use_dense_path() else _HMatFunction
+            if U.dtype != torch.float32:
+                U = U.float()
+            if U.stride(1) != 1:
+                U = U.contiguous()
         anchor = self.__dict__.get("_dev_anchor")
         if anchor is None or anchor.device != U.device:
             anchor = torch.zeros(1, device=U.device, requires_grad=True)
             self.__dict__["_dev_anchor"] = anchor
         needs = torch.is_grad_enabled() and self._nleaves > 0
-        fn = _HMatDenseFunction if self._use_dense_path() else _HMatFunction
         return fn.apply(U, anchor if needs else None, self)
 
     def get_nb_parameters(self) -> int:

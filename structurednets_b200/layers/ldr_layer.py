@@ -15,6 +15,7 @@ import torch
 import torch.nn as nn
 
 from structurednets_b200 import _lib
+from structurednets_b200.layers import dense_bf16 as D
 from structurednets_b200.layers.layer_helpers import get_random_glorot_uniform_matrix_torch
 from structurednets_b200.layers.structured_layer import StructuredLayer
 
@@ -72,42 +73,63 @@ def band_slots(indices: torch.Tensor, n: int) -> torch.Tensor:
     return slot.to(torch.int32).contiguous()
 
 
-class _LDRFunction(torch.autograd.Function):
-    """sn_ldr_build_weight + sn_dense_apply / sn_dense_weight_grad + sn_ldr_backward (csrc/ldr_tl.cu).  Nothing on this path
+def _ldr_build_weight(layer, dev, A, Bm, G, H):
+    """W (n x n, float32) from the representation, with the workspace, status word and term count the backward needs.  Nothing here
     synchronises while a CUDA graph is being captured; outside a capture the 16-byte status word is read back after the Krylov
     kernels so that a series longer than the powers computed is re-run with more (and ``last_nb_terms`` stays observable)."""
+    n, r = G.shape
+    L = _lib.lib()
+    slots = layer._slots(A, Bm)
+    Av, Bv = A._values().contiguous(), Bm._values().contiguous()
+    Gc, Hc = G.contiguous(), H.contiguous()
+    assert Av.dtype == torch.float64 and Gc.dtype == torch.float64, "LDR representation matrices are float64 (SURVEY.md F4)"
+    W = torch.empty((n, n), dtype=torch.float32, device=dev)
+    status = torch.zeros(4, dtype=torch.int32, device=dev)
+    capturing = torch.cuda.is_current_stream_capturing()
+    max_terms = min(n, 1024, int(layer.__dict__.get("_terms_cap", LDR_TERMS_START)))
+    while True:
+        ws = torch.empty(int(L.sn_ldr_workspace_bytes(n, r, max_terms)), dtype=torch.uint8, device=dev)
+        rc = L.sn_ldr_build_weight(n, r, _lib.ptr(Av), _lib.ptr(slots[0]), Av.numel(), _lib.ptr(Bv), _lib.ptr(slots[1]), Bv.numel(),
+                                   _lib.ptr(Gc), _lib.ptr(Hc), _lib.ptr(ws), max_terms, LDR_REL_TOL, _lib.ptr(W), _lib.ptr(status), _lib.stream_ptr())
+        _lib.check(rc, "sn_ldr_build_weight")
+        if capturing:
+            break
+        st = status.tolist()
+        layer.last_nb_terms = int(st[0])
+        if st[2] or max_terms >= min(n, 1024):
+            if st[2]:   # next call computes a few powers more than this one needed, not LDR_TERMS_START
+                layer.__dict__["_terms_cap"] = min(n, 1024, max(8, (int(st[0]) + 4 + 3) // 4 * 4))
+            if not st[2]:
+                raise RuntimeError("LDRLayer: the Krylov series of this (A, B) has not decayed after %d powers (n = %d); the operators' "
+                                   "norms are too close to (or above) 1 for the truncated construction" % (max_terms, n))
+            break
+        max_terms = min(n, 1024, max_terms * 4)
+        layer.__dict__["_terms_cap"] = max_terms
+    return W, ws, status, max_terms, slots, Gc, Hc
+
+
+def _ldr_param_grads(dW, slots, ws, max_terms, status, A, Bm, G, H):
+    """dW -> sparse dA, dB on the parameters' own pattern (SURVEY.md F4) and dense dG, dH, all float64."""
+    n, r = G.shape
+    dev = dW.device
+    gA = torch.zeros(A._nnz(), dtype=torch.float64, device=dev)
+    gB = torch.zeros(Bm._nnz(), dtype=torch.float64, device=dev)
+    gG, gH = torch.zeros_like(G), torch.zeros_like(H)
+    rc = _lib.lib().sn_ldr_backward(n, r, _lib.ptr(dW), _lib.ptr(slots[0]), gA.numel(), _lib.ptr(slots[1]), gB.numel(), _lib.ptr(ws),
+                                    max_terms, _lib.ptr(status), _lib.ptr(gA), _lib.ptr(gB), _lib.ptr(gG), _lib.ptr(gH), _lib.stream_ptr())
+    _lib.check(rc, "sn_ldr_backward")
+    return torch.sparse_coo_tensor(A._indices(), gA, A.shape), torch.sparse_coo_tensor(Bm._indices(), gB, Bm.shape), gG, gH
+
+
+class _LDRFunction(torch.autograd.Function):
+    """sn_ldr_build_weight + sn_dense_apply / sn_dense_weight_grad + sn_ldr_backward (csrc/ldr_tl.cu), see _ldr_build_weight."""
 
     @staticmethod
     def forward(ctx, U, bias, layer, A, Bm, G, H):
         n, r = G.shape
         dev = U.device
         L = _lib.lib()
-        slots = layer._slots(A, Bm)
-        Av, Bv = A._values().contiguous(), Bm._values().contiguous()
-        Gc, Hc = G.contiguous(), H.contiguous()
-        assert Av.dtype == torch.float64 and Gc.dtype == torch.float64, "LDR representation matrices are float64 (SURVEY.md F4)"
-        W = torch.empty((n, n), dtype=torch.float32, device=dev)
-        status = torch.zeros(4, dtype=torch.int32, device=dev)
-        capturing = torch.cuda.is_current_stream_capturing()
-        max_terms = min(n, 1024, int(layer.__dict__.get("_terms_cap", LDR_TERMS_START)))
-        while True:
-            ws = torch.empty(int(L.sn_ldr_workspace_bytes(n, r, max_terms)), dtype=torch.uint8, device=dev)
-            rc = L.sn_ldr_build_weight(n, r, _lib.ptr(Av), _lib.ptr(slots[0]), Av.numel(), _lib.ptr(Bv), _lib.ptr(slots[1]), Bv.numel(),
-                                       _lib.ptr(Gc), _lib.ptr(Hc), _lib.ptr(ws), max_terms, LDR_REL_TOL, _lib.ptr(W), _lib.ptr(status), _lib.stream_ptr())
-            _lib.check(rc, "sn_ldr_build_weight")
-            if capturing:
-                break
-            st = status.tolist()
-            layer.last_nb_terms = int(st[0])
-            if st[2] or max_terms >= min(n, 1024):
-                if st[2]:   # next call computes a few powers more than this one needed, not LDR_TERMS_START
-                    layer.__dict__["_terms_cap"] = min(n, 1024, max(8, (int(st[0]) + 4 + 3) // 4 * 4))
-                if not st[2]:
-                    raise RuntimeError("LDRLayer: the Krylov series of this (A, B) has not decayed after %d powers (n = %d); the operators' "
-                                       "norms are too close to (or above) 1 for the truncated construction" % (max_terms, n))
-                break
-            max_terms = min(n, 1024, max_terms * 4)
-            layer.__dict__["_terms_cap"] = max_terms
+        W, ws, status, max_terms, slots, Gc, Hc = _ldr_build_weight(layer, dev, A, Bm, G, H)
         y = torch.empty((U.shape[0], n), dtype=torch.float32, device=dev)
         rc = L.sn_dense_apply(_lib.ptr(W), n, n, _lib.ptr(U), U.stride(0), _lib.ptr(y), y.stride(0), _lib.ptr(bias), U.shape[0], _lib.stream_ptr())
         _lib.check(rc, "sn_dense_apply")
@@ -132,14 +154,32 @@ class _LDRFunction(torch.autograd.Function):
         rc = L.sn_dense_weight_grad(_lib.ptr(U), U.stride(0), _lib.ptr(grad_y), grad_y.stride(0), _lib.ptr(dW), n, n, _lib.ptr(gbias),
                                     U.shape[0], _lib.stream_ptr())
         _lib.check(rc, "sn_dense_weight_grad")
-        gA = torch.zeros(A._nnz(), dtype=torch.float64, device=dev)
-        gB = torch.zeros(Bm._nnz(), dtype=torch.float64, device=dev)
-        gG, gH = torch.zeros_like(G), torch.zeros_like(H)
-        rc = L.sn_ldr_backward(n, r, _lib.ptr(dW), _lib.ptr(ctx.slots[0]), gA.numel(), _lib.ptr(ctx.slots[1]), gB.numel(), _lib.ptr(ws),
-                               ctx.max_terms, _lib.ptr(status), _lib.ptr(gA), _lib.ptr(gB), _lib.ptr(gG), _lib.ptr(gH), _lib.stream_ptr())
-        _lib.check(rc, "sn_ldr_backward")
-        gAs = torch.sparse_coo_tensor(A._indices(), gA, A.shape)   # sparse grads on the parameters' own pattern (SURVEY.md F4)
-        gBs = torch.sparse_coo_tensor(Bm._indices(), gB, Bm.shape)
+        gAs, gBs, gG, gH = _ldr_param_grads(dW, ctx.slots, ws, ctx.max_terms, status, A, Bm, G, H)
+        return grad_x, gbias, None, gAs, gBs, gG, gH
+
+
+class _LDRBF16Function(torch.autograd.Function):
+    """bfloat16 features: the same float32 W, applied and differentiated on bf16 tensor cores (layers/dense_bf16.py)."""
+
+    @staticmethod
+    def forward(ctx, U, bias, layer, A, Bm, G, H):
+        W, ws, status, max_terms, slots, Gc, Hc = _ldr_build_weight(layer, U.device, A, Bm, G, H)
+        x = D.staged(U)
+        y, Wtb = D.forward(layer, W, x, bias, keep_wt=ctx.needs_input_grad[0])
+        ctx.max_terms, ctx.slots, ctx.has_bias = max_terms, slots, bias is not None
+        ctx.save_for_backward(x, ws, status, Wtb, A, Bm, Gc, Hc)
+        return y
+
+    @staticmethod
+    def backward(ctx, grad_y):
+        x, ws, status, Wtb, A, Bm, G, H = ctx.saved_tensors
+        n = G.shape[0]
+        gy = D.staged(grad_y)
+        grad_x = D.input_grad(Wtb, gy) if ctx.needs_input_grad[0] else None
+        dW = torch.zeros((n, n), dtype=torch.float32, device=x.device)
+        gbias = torch.zeros(n, dtype=torch.float32, device=x.device) if ctx.has_bias else None
+        D.weight_grad(x, gy, dW, gbias)
+        gAs, gBs, gG, gH = _ldr_param_grads(dW, ctx.slots, ws, ctx.max_terms, status, A, Bm, G, H)
         return grad_x, gbias, None, gAs, gBs, gG, gH
 
 
@@ -187,6 +227,7 @@ class LDRLayer(StructuredLayer):
     def __getstate__(self):
         state = self.__dict__.copy()
         state.pop("_dev_slots", None)
+        state.pop("_dev_W_bf16", None)
         return state
 
     def forward(self, U):
@@ -194,6 +235,8 @@ class LDRLayer(StructuredLayer):
             return torch.zeros((U.shape[0], self.output_dim), device=U.device)   # reference ldr_layer.py:51-52
         self._require_cuda(U, "LDRLayer.forward")
         assert U.dim() == 2 and U.shape[1] == self.input_dim, "LDRLayer expects a (batch, input_dim) input"
+        if U.dtype == torch.bfloat16:     # bf16 output, float32 / float64 parameters and gradients
+            return _LDRBF16Function.apply(U, self.bias if self.use_bias else None, self, *self.representation_matrices)
         if U.dtype != torch.float32:
             U = U.float()
         if U.stride(1) != 1:

@@ -16,6 +16,7 @@ import torch
 import torch.nn as nn
 
 from structurednets_b200 import _lib
+from structurednets_b200.layers import dense_bf16 as D
 from structurednets_b200.layers.layer_helpers import get_random_glorot_uniform_matrix
 from structurednets_b200.layers.structured_layer import StructuredLayer
 
@@ -141,6 +142,48 @@ class _PSMDenseFunction(torch.autograd.Function):
         return (grad_x, gbias, None, *gf)
 
 
+class _PSMDenseBF16Function(torch.autograd.Function):
+    """bfloat16 features: the dense-product path's prefix products and projection, the batch GEMMs on bf16 tensor cores
+    (sn_psm_dense_forward_bf16 / sn_psm_dense_backward_bf16, layers/dense_bf16.py)."""
+
+    @staticmethod
+    def forward(ctx, U, bias, layer, *factors):
+        patterns = layer._dense_patterns(factors)
+        assert all(p._values().dtype == torch.float32 and p._values().is_contiguous() for p in factors)
+        arr = _dense_factor_array(patterns, factors, None)
+        L = _lib.lib()
+        x = D.staged(U)
+        B, dev = x.shape[0], x.device
+        prefix = torch.empty(L.sn_psm_dense_prefix_floats(arr, len(factors), layer.output_dim), dtype=torch.float32, device=dev)
+        Wb = D.weight_buffer(layer, layer.output_dim, layer.input_dim, dev)
+        Wtb = torch.empty((layer.input_dim, D.pad8(layer.output_dim)), dtype=torch.bfloat16, device=dev) if ctx.needs_input_grad[0] else None
+        y = D.empty_rows(B, layer.output_dim, dev)
+        rc = L.sn_psm_dense_forward_bf16(arr, len(factors), _lib.ptr(x), x.stride(0), _lib.ptr(y), y.stride(0), _lib.ptr(bias), _lib.ptr(prefix),
+                                         _lib.ptr(Wb), Wb.stride(0), _lib.ptr(Wtb), Wtb.stride(0) if Wtb is not None else 0, B, layer.input_dim,
+                                         layer.output_dim, _lib.stream_ptr())
+        _lib.check(rc, "sn_psm_dense_forward_bf16")
+        ctx.layer, ctx.patterns, ctx.has_bias = layer, patterns, bias is not None
+        ctx.save_for_backward(x, prefix, Wtb, *factors)
+        return y
+
+    @staticmethod
+    def backward(ctx, grad_y):
+        x, prefix, Wtb, *factors = ctx.saved_tensors
+        layer = ctx.layer
+        gy = D.staged(grad_y)
+        gvals = [torch.zeros(p._nnz(), dtype=torch.float32, device=x.device) for p in factors]
+        gbias = torch.zeros(layer.output_dim, dtype=torch.float32, device=x.device) if ctx.has_bias else None
+        arr = _dense_factor_array(ctx.patterns, factors, gvals)
+        L = _lib.lib()
+        work = torch.empty(L.sn_psm_dense_backward_floats(arr, len(factors), layer.output_dim), dtype=torch.float32, device=x.device)
+        rc = L.sn_psm_dense_backward_bf16(arr, len(factors), _lib.ptr(x), x.stride(0), _lib.ptr(gy), gy.stride(0), _lib.ptr(prefix), _lib.ptr(work),
+                                          _lib.ptr(gbias), x.shape[0], layer.input_dim, layer.output_dim, _lib.stream_ptr())
+        _lib.check(rc, "sn_psm_dense_backward_bf16")
+        grad_x = D.input_grad(Wtb, gy) if ctx.needs_input_grad[0] else None
+        gf = [torch.sparse_coo_tensor(p._indices(), g, p.shape) for p, g in zip(factors, gvals)]
+        return (grad_x, gbias, None, *gf)
+
+
 def _factor_array(patterns, params, gvals):
     arr = (_lib.SnPsmFactor * len(params))()
     for k, (pat, p) in enumerate(zip(patterns, params)):
@@ -260,7 +303,7 @@ class PSMLayer(StructuredLayer):
         SNB200_PSM_PATH=dense|sparse forces a path."""
         import os
         forced = os.environ.get("SNB200_PSM_PATH", "")
-        eligible = self.output_dim % 4 == 0 and max(max(p.shape) for p in self.sparse_matrices) <= 16384
+        eligible = self._dense_eligible()
         if forced == "dense":
             assert eligible, "PSMLayer: the dense-product path needs output_dim % 4 == 0 and factor dimensions <= 16384"
             return True
@@ -268,18 +311,29 @@ class PSMLayer(StructuredLayer):
             return False
         return eligible and batch >= 1024
 
+    def _dense_eligible(self) -> bool:
+        return self.output_dim % 4 == 0 and max(max(p.shape) for p in self.sparse_matrices) <= 16384
+
+    def use_dense_bf16_path(self) -> bool:
+        """bfloat16 features take the dense-product path on bf16 tensor cores whenever the layer is eligible for it and
+        SNB200_PSM_PATH does not force the sparse chain -- at every batch size, so the output dtype does not depend on the batch."""
+        import os
+        return os.environ.get("SNB200_PSM_PATH", "") != "sparse" and self._dense_eligible()
+
     def __getstate__(self):
         state = self.__dict__.copy()
         state.pop("_dev_patterns", None)
         state.pop("_dev_dense_patterns", None)
+        state.pop("_dev_W_bf16", None)
         return state
 
     def forward(self, U):
         self._require_cuda(U, "PSMLayer.forward")
         assert U.dim() == 2 and U.shape[1] == self.input_dim, "PSMLayer expects a (batch, input_dim) input"
-        if U.dtype != torch.float32:
+        bf16 = U.dtype == torch.bfloat16 and self.use_dense_bf16_path()    # bf16 output, float32 parameters and gradients
+        if not bf16 and U.dtype != torch.float32:
             U = U.float()
-        if U.stride(1) != 1:
+        if not bf16 and U.stride(1) != 1:
             U = U.contiguous()
         # torch's sparse SGD update on CUDA (param.add_(sparse_grad)) concatenates the indices instead of summing
         # matching entries, so nnz grows with every step; fold duplicates back before using the pattern.
@@ -288,7 +342,10 @@ class PSMLayer(StructuredLayer):
                 with torch.no_grad():
                     p.data = p.detach().coalesce()
                 self._base_nnz[k] = int(p._nnz())
-        fn = _PSMDenseFunction if self.use_dense_path(U.shape[0]) else _PSMFunction
+        if bf16:
+            fn = _PSMDenseBF16Function
+        else:
+            fn = _PSMDenseFunction if self.use_dense_path(U.shape[0]) else _PSMFunction
         return fn.apply(U, self.bias if self.use_bias else None, self, *self.sparse_matrices)
 
     forward_sparse = forward   # the reference's alternative torch.sparse.mm path (psm_layer.py:36-45): same math

@@ -10,10 +10,31 @@ import torch
 import torch.nn as nn
 
 from structurednets_b200 import _lib
+from structurednets_b200.layers import dense_bf16 as D
 from structurednets_b200.layers.flat_params import FlatParamsMixin
 from structurednets_b200.layers.layer_helpers import get_random_glorot_uniform_matrix
 from structurednets_b200.layers.lr_layer import svd_low_rank_factors
 from structurednets_b200.layers.structured_layer import StructuredLayer
+
+
+def _tl_build_weight(layer, dev):
+    """W (n x n, float32) and the Krylov scratch K1, K2 that sn_tl_backward reuses."""
+    n, r = layer.G.shape
+    K1 = torch.empty((n, n * r), dtype=torch.float32, device=dev)
+    K2 = torch.empty((n * r, n), dtype=torch.float32, device=dev)
+    W = torch.empty((n, n), dtype=torch.float32, device=dev)
+    rc = _lib.lib().sn_tl_build_weight(n, r, _lib.ptr(layer.G), _lib.ptr(layer.H), _lib.ptr(K1), _lib.ptr(K2), _lib.ptr(W), _lib.stream_ptr())
+    _lib.check(rc, "sn_tl_build_weight")
+    return W, K1, K2
+
+
+def _tl_param_grads(layer, dW, K1, K2):
+    """dW -> G.grad, H.grad (accumulated into the flat gradient buffer)."""
+    n, r = layer.G.shape
+    dK1, dK2 = torch.empty_like(K1), torch.empty_like(K2)
+    rc = _lib.lib().sn_tl_backward(n, r, _lib.ptr(dW), _lib.ptr(K1), _lib.ptr(K2), _lib.ptr(dK1), _lib.ptr(dK2), _lib.ptr(layer.G.grad),
+                                   _lib.ptr(layer.H.grad), _lib.stream_ptr())
+    _lib.check(rc, "sn_tl_backward")
 
 
 class _TLFunction(torch.autograd.Function):
@@ -21,11 +42,7 @@ class _TLFunction(torch.autograd.Function):
     def forward(ctx, U, anchor, layer):
         n, r = layer.G.shape
         dev = U.device
-        K1 = torch.empty((n, n * r), dtype=torch.float32, device=dev)
-        K2 = torch.empty((n * r, n), dtype=torch.float32, device=dev)
-        W = torch.empty((n, n), dtype=torch.float32, device=dev)
-        rc = _lib.lib().sn_tl_build_weight(n, r, _lib.ptr(layer.G), _lib.ptr(layer.H), _lib.ptr(K1), _lib.ptr(K2), _lib.ptr(W), _lib.stream_ptr())
-        _lib.check(rc, "sn_tl_build_weight")
+        W, K1, K2 = _tl_build_weight(layer, dev)
         y = torch.empty((U.shape[0], n), dtype=torch.float32, device=dev)
         rc = _lib.lib().sn_dense_apply(_lib.ptr(W), n, n, _lib.ptr(U), U.stride(0), _lib.ptr(y), y.stride(0),
                                        _lib.ptr(layer.bias if layer.use_bias else None), U.shape[0], _lib.stream_ptr())
@@ -52,10 +69,33 @@ class _TLFunction(torch.autograd.Function):
         rc = _lib.lib().sn_dense_weight_grad(_lib.ptr(U), U.stride(0), _lib.ptr(grad_y), grad_y.stride(0), _lib.ptr(dW), n, n, _lib.ptr(gb),
                                              U.shape[0], _lib.stream_ptr())
         _lib.check(rc, "sn_dense_weight_grad")
-        dK1, dK2 = torch.empty_like(K1), torch.empty_like(K2)
-        rc = _lib.lib().sn_tl_backward(n, r, _lib.ptr(dW), _lib.ptr(K1), _lib.ptr(K2), _lib.ptr(dK1), _lib.ptr(dK2), _lib.ptr(layer.G.grad),
-                                       _lib.ptr(layer.H.grad), _lib.stream_ptr())
-        _lib.check(rc, "sn_tl_backward")
+        _tl_param_grads(layer, dW, K1, K2)
+        return grad_x, None, None
+
+
+class _TLBF16Function(torch.autograd.Function):
+    """bfloat16 features: the same float32 W, applied and differentiated on bf16 tensor cores (layers/dense_bf16.py)."""
+
+    @staticmethod
+    def forward(ctx, U, anchor, layer):
+        W, K1, K2 = _tl_build_weight(layer, U.device)
+        x = D.staged(U)
+        y, Wtb = D.forward(layer, W, x, layer.bias if layer.use_bias else None, keep_wt=ctx.needs_input_grad[0])
+        ctx.layer = layer
+        ctx.save_for_backward(x, K1, K2, Wtb)
+        return y
+
+    @staticmethod
+    def backward(ctx, grad_y):
+        layer = ctx.layer
+        x, K1, K2, Wtb = ctx.saved_tensors
+        n = layer.G.shape[0]
+        gy = D.staged(grad_y)
+        grad_x = D.input_grad(Wtb, gy) if ctx.needs_input_grad[0] else None
+        layer._prepare_grad_accumulation()
+        dW = torch.zeros((n, n), dtype=torch.float32, device=x.device)
+        D.weight_grad(x, gy, dW, layer.bias.grad if (layer.use_bias and layer.bias.requires_grad) else None)
+        _tl_param_grads(layer, dW, K1, K2)
         return grad_x, None, None
 
 
@@ -93,15 +133,19 @@ class TLLayer(FlatParamsMixin, StructuredLayer):
             self._require_cuda(U, "TLLayer.forward")
             assert U.dim() == 2 and U.shape[1] == self.input_dim, "TLLayer expects a (batch, input_dim) input"
             self._ensure_flat()
-            if U.dtype != torch.float32:
-                U = U.float()
-            if U.stride(1) != 1:
-                U = U.contiguous()
+            if U.dtype == torch.bfloat16:     # bf16 output, float32 parameters and gradients
+                fn = _TLBF16Function
+            else:
+                fn = _TLFunction
+                if U.dtype != torch.float32:
+                    U = U.float()
+                if U.stride(1) != 1:
+                    U = U.contiguous()
             anchor = self.__dict__.get("_dev_anchor")
             if anchor is None or anchor.device != U.device:
                 anchor = torch.zeros(1, device=U.device, requires_grad=True)
                 self.__dict__["_dev_anchor"] = anchor
-            return _TLFunction.apply(U, anchor if torch.is_grad_enabled() else None, self)
+            return fn.apply(U, anchor if torch.is_grad_enabled() else None, self)
         y_pred = torch.zeros((U.shape[0], self.output_dim), device=U.device)   # reference tl_layer.py:62-63
         if self.use_bias:
             y_pred = y_pred + self.bias
