@@ -94,8 +94,10 @@ int sn_sss_pack(const sn_sss_plan* plan_host, const float* params, float* packed
 int sn_sss_forward(const sn_sss_plan* plan_host, const float* packed, const float* x, int64_t ldx,
                    float* y, int64_t ldy, const float* bias, float* ckpt, int64_t B, sn_stream_t stream);
 /* grad_params (flat, same layout as params) += d loss / d params ; grad_bias (may be NULL) += column
- * sums of grad_y.  grad_x (may be NULL) receives d loss / d x (overwritten).  workspace: scratch of
- * sn_sss_backward_workspace_floats() floats (packed per-stage gradient accumulators). */
+ * sums of grad_y.  grad_x (may be NULL; row stride ldgx >= input_dim) receives d loss / d x (overwritten,
+ * bitwise reproducible).  workspace: scratch of sn_sss_backward_workspace_floats() floats (packed per-stage
+ * gradient accumulators).  grad_params may be NULL when grad_x is not (input gradient only, e.g. frozen
+ * parameters); workspace may then be NULL too.  grad_params and grad_x both NULL is an error. */
 size_t sn_sss_backward_workspace_floats(const sn_sss_plan* plan_host);
 int sn_sss_backward(const sn_sss_plan* plan_host, const float* packed, const float* x, int64_t ldx,
                     const float* grad_y, int64_t ldgy, const float* ckpt, float* workspace, float* grad_params,
@@ -146,6 +148,8 @@ int sn_sss_tc_backward(const sn_sss_tc_plan* plan_host, const float* params, con
                        const float* grad_y, int64_t ldgy, const float* states, float* workspace, float* grad_params, float* grad_bias,
                        float* grad_x /* nullable: gradient w.r.t. the input features, (B x input_dim), written */, int64_t ldgx,
                        int64_t B, sn_stream_t stream);
+/* sn_sss_tc_backward: grad_params may be NULL when grad_x is not (input gradient only: the scans and the grad_x products run, the
+ * parameter-gradient kernels do not; grad_bias is still accumulated when given).  Both NULL is an error.  workspace is always needed. */
 
 /* ------------------------------------------------------------------------------------------
  * Low-rank layer, fp32 path -- replaces LRLayer.forward (layers/lr_layer.py:38-46) and its backward.

@@ -496,9 +496,14 @@ sss_fwd_kernel(sn_sss_plan plan, const float* __restrict__ packed, const float* 
 //             chunk's adjoint sweep has released the parameter buffer, i.e. it lands during the gradient phase
 //   1. recompute the entry states of the chunk's stages                         (warp-own samples)
 //   2. adjoint sweep  lam_in = P^T [lam_out ; gy]                               (warp-own samples)
+//   2b. (grad_x only) input gradients  grad_u = the in_dim input columns of P^T [lam_out ; gy]  (own samples, all
+//      lanes), staged per stage in a per-warp [column][position] buffer and added to grad_x with coalesced
+//      red.global.add: each direction adds its share exactly once onto the zeroed grad_x, so the sum of the two
+//      addends is bitwise reproducible.  Runs before the parameter buffer is handed back to the bulk copy.
 //   3. parameter gradients  dP_k = [lam_out ; gy] [s_in ; u]^T over the tile's samples (warp-own stages,
 //      4x4 register tiles over interleaved rows/cols), atomically accumulated into a packed [r][k_pad]
 //      gradient workspace that sss_unpack_grad_kernel folds into the flat gradient buffer afterwards.
+//      Skipped when only grad_x is requested (gpacked == NULL).
 // ------------------------------------------------------------------------------------------
 constexpr int BWD_CONS = 2;
 constexpr int BWD_THREADS = BWD_CONS * 32;
@@ -507,10 +512,13 @@ struct BwdSmem {
     int nsp;     // padded position stride of the CTA-wide feature-major buffers
     int blk;     // floats per packed stage block
     int hs;      // one history entry (d_pad * nsp)
-    int params, bars, pos, xh, lh, lcar0, lcar1, ck0, ck1, ut0, ut1, gt0, gt1, zero, total;   // float offsets
+    int gxs;     // position stride of the grad_u staging buffer (0: no grad_x)
+    int params, bars, pos, xh, lh, lcar0, lcar1, ck0, ck1, ut0, ut1, gt0, gt1, zero, gx, total;   // float offsets
 };
 
-inline BwdSmem make_bwd_smem(const sn_sss_plan& p, const Geom& g) {
+// with_gx: add the per-warp grad_u staging buffer (one stage's input columns; every stage lies in one half chunk, so half_in_max
+// bounds its in_dim).  Without it the layout is exactly that of a parameter-gradient-only backward.
+inline BwdSmem make_bwd_smem(const sn_sss_plan& p, const Geom& g, bool with_gx) {
     BwdSmem s;
     const int ns = BWD_CONS * g.nsw;
     s.nsp = pad_stride(ns);
@@ -532,6 +540,8 @@ inline BwdSmem make_bwd_smem(const sn_sss_plan& p, const Geom& g) {
     s.gt0 = o;    o += p.chunk_out_max * s.nsp;
     s.gt1 = o;    o += p.chunk_out_max * s.nsp;
     s.zero = o;   o += s.nsp;
+    s.gxs = with_gx ? pad_stride(g.nsw) : 0;
+    s.gx = o;     o += with_gx ? BWD_CONS * p.half_in_max * s.gxs : 0;
     s.total = o;
     return s;
 }
@@ -580,7 +590,7 @@ template <int RP4T, int KP4T, int NSPT>
 __global__ void __launch_bounds__(BWD_THREADS)
 sss_bwd_kernel(sn_sss_plan plan, const float* __restrict__ packed, const float* __restrict__ x, long ldx,
                const float* __restrict__ gy, long ldgy, const float* __restrict__ ckpt,
-               float* __restrict__ gpacked, float* __restrict__ gbias, long B, Geom g, BwdSmem sm) {
+               float* __restrict__ gpacked, float* __restrict__ gbias, float* __restrict__ gx, long ldgx, long B, Geom g, BwdSmem sm) {
     extern __shared__ __align__(128) float smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int dir = blockIdx.y;
@@ -747,6 +757,57 @@ sss_bwd_kernel(sn_sss_plan plan, const float* __restrict__ packed, const float* 
             }
             __syncwarp();
         }
+        // ---- 2b. input gradients (own samples, all lanes; off the recurrence) ---------------------
+        if (gx != nullptr) {
+            float* gxb = smem + sm.gx + (size_t)warp * plan.half_in_max * sm.gxs;
+            for (int j = 0; j < len; ++j) {
+                const float* slot = params + (size_t)j * sm.blk;
+                const int* hdr = reinterpret_cast<const int*>(slot);
+                const int in_off = hdr[0], in_dim = hdr[1], out_off = hdr[2], out_dim = hdr[3], d_in = hdr[4], d_out = hdr[5];
+                const float4* P4 = reinterpret_cast<const float4*>(slot + SSS_HDR + KP * RP);
+                const float* lout = (j == len - 1 ? lcar_cur : lh + (size_t)j * hs) + w0;
+                const float* gyj = gt + (size_t)(out_off - c.row0) * NSP + w0;
+                // aligned 4-column groups covering the input columns [d_in, d_in + in_dim) of P
+                const int cg0 = d_in >> 2, ncg = ((d_in + in_dim + 3) >> 2) - cg0;
+                for (int t = lane; t < ncg * nq; t += 32) {
+                    const int cg = cg0 + t / nq, qq = t % nq;
+                    float acc[4][4];
+#pragma unroll
+                    for (int a = 0; a < 4; ++a)
+#pragma unroll
+                        for (int b = 0; b < 4; ++b) acc[a][b] = 0.f;
+                    const float4* prow = P4 + cg;
+                    const float* lv = lout + 4 * qq;
+#pragma unroll 4
+                    for (int r = 0; r < d_out; ++r) {
+                        const float4 p = prow[0];
+                        const float4 v = *reinterpret_cast<const float4*>(lv);
+                        prow += KP4; lv += NSP;
+                        fma16(acc, p, v);
+                    }
+                    const float* gv = gyj + 4 * qq;
+                    for (int r = 0; r < out_dim; ++r) {
+                        const float4 p = prow[0];
+                        const float4 v = *reinterpret_cast<const float4*>(gv);
+                        prow += KP4; gv += NSP;
+                        fma16(acc, p, v);
+                    }
+#pragma unroll
+                    for (int a = 0; a < 4; ++a) {
+                        const int cc = 4 * cg + a - d_in;
+                        if (cc >= 0 && cc < in_dim)
+                            *reinterpret_cast<float4*>(gxb + cc * sm.gxs + 4 * qq) = make_float4(acc[a][0], acc[a][1], acc[a][2], acc[a][3]);
+                    }
+                }
+                __syncwarp();
+                // lanes along the stage's contiguous columns of consecutive samples
+                for (int e = lane; e < nvalid * in_dim; e += 32) {
+                    const int ls = e / in_dim, cc = e - ls * in_dim;
+                    atomicAdd(gx + (size_t)(samp0 + ls) * ldgx + in_off + cc, gxb[cc * sm.gxs + ls]);
+                }
+                __syncwarp();
+            }
+        }
         // stage descriptors needed by the gradient phase are copied out before the parameter buffer is released
         int h_in_off[2], h_in_dim[2], h_out_off[2], h_out_dim[2], h_d_in[2], h_d_out[2];
 #pragma unroll
@@ -785,7 +846,7 @@ sss_bwd_kernel(sn_sss_plan plan, const float* __restrict__ packed, const float* 
 #pragma unroll
         for (int u = 0; u < 2; ++u) {            // chunk_len_max <= 2*BWD_CONS is checked on the host
             const int j = warp + u * BWD_CONS;
-            if (j >= len) break;
+            if (j >= len || gpacked == nullptr) break;
             const int in_off = h_in_off[u], in_dim = h_in_dim[u], out_off = h_out_off[u], out_dim = h_out_dim[u], d_in = h_d_in[u], d_out = h_d_out[u];
             const int rows = d_out + out_dim, K = d_in + in_dim;
             const int rgn = (rows + 3) >> 2, cgn = (K + 3) >> 2;
@@ -958,28 +1019,33 @@ int sn_sss_backward(const sn_sss_plan* p, const float* packed, const float* x, i
                     int64_t ldgy, const float* ckpt, float* workspace, float* grad_params, float* grad_bias, float* grad_x,
                     int64_t ldgx, int64_t B, sn_stream_t stream) {
     if (int rc = check_plan(p)) return rc;
-    (void)ldgx;
-    SN_CHECK_ARG(packed && x && grad_y && ckpt && grad_params && workspace, "sss_backward: NULL buffer");
-    SN_CHECK_ARG(grad_x == nullptr, "sss_backward: grad_x is not implemented (the reference training loop never needs it)");
+    SN_CHECK_ARG(packed && x && grad_y && ckpt, "sss_backward: NULL buffer");
+    SN_CHECK_ARG(grad_params != nullptr || grad_x != nullptr, "sss_backward: grad_params and grad_x are both NULL (nothing to compute)");
+    SN_CHECK_ARG(grad_params == nullptr || workspace != nullptr, "sss_backward: NULL workspace");
     SN_CHECK_ARG(ldx >= p->input_dim && ldgy >= p->output_dim, "sss_backward: leading dimension too small");
+    SN_CHECK_ARG(grad_x == nullptr || ldgx >= p->input_dim, "sss_backward: grad_x leading dimension too small");
     if (B <= 0) return 0;
     cudaStream_t st = snb::as_stream(stream);
     Geom g = make_geom(p->rows_pad);
-    BwdSmem sm = make_bwd_smem(*p, g);
+    BwdSmem sm = make_bwd_smem(*p, g, grad_x != nullptr);
     size_t smem = (size_t)sm.total * sizeof(float);
     SN_CHECK_ARG(smem <= 227 * 1024, "sss_backward: stage dims need %zu bytes of shared memory (> 227 KB)", smem);
     SN_CHECK_ARG(p->chunk_len_max <= 2 * BWD_CONS, "sss_backward: chunks of more than %d stages are not supported", 2 * BWD_CONS);
     const bool fast = p->rows_pad == 20 && p->k_pad == 28 && sm.nsp == 52 && g.nsw == 24;
     SN_SET_MAX_SMEM(227 * 1024, sss_bwd_kernel<5, 7, 52>);
     SN_SET_MAX_SMEM(227 * 1024, sss_bwd_kernel<0, 0, 0>);
-    SN_CHECK_CUDA(cudaMemsetAsync(workspace, 0, sn_sss_backward_workspace_floats(p) * sizeof(float), st));
+    if (grad_params != nullptr) SN_CHECK_CUDA(cudaMemsetAsync(workspace, 0, sn_sss_backward_workspace_floats(p) * sizeof(float), st));
+    // both directions add their share of grad_x onto zero (two addends per element: the sum does not depend on their order)
+    if (grad_x != nullptr) SN_CHECK_CUDA(cudaMemset2DAsync(grad_x, (size_t)ldgx * sizeof(float), 0, (size_t)p->input_dim * sizeof(float), (size_t)B, st));
+    float* gpacked = grad_params != nullptr ? workspace : nullptr;
     long tile = (long)BWD_CONS * g.nsw;
     dim3 grid((unsigned)((B + tile - 1) / tile), 2);
     snb::timing_begin("sss_bwd_kernel", st);
-    if (fast) sss_bwd_kernel<5, 7, 52><<<grid, BWD_THREADS, smem, st>>>(*p, packed, x, (long)ldx, grad_y, (long)ldgy, ckpt, workspace, grad_bias, (long)B, g, sm);
-    else sss_bwd_kernel<0, 0, 0><<<grid, BWD_THREADS, smem, st>>>(*p, packed, x, (long)ldx, grad_y, (long)ldgy, ckpt, workspace, grad_bias, (long)B, g, sm);
+    if (fast) sss_bwd_kernel<5, 7, 52><<<grid, BWD_THREADS, smem, st>>>(*p, packed, x, (long)ldx, grad_y, (long)ldgy, ckpt, gpacked, grad_bias, grad_x, (long)ldgx, (long)B, g, sm);
+    else sss_bwd_kernel<0, 0, 0><<<grid, BWD_THREADS, smem, st>>>(*p, packed, x, (long)ldx, grad_y, (long)ldgy, ckpt, gpacked, grad_bias, grad_x, (long)ldgx, (long)B, g, sm);
     snb::timing_end(st);
     SN_CHECK_LAUNCH("sss_bwd_kernel");
+    if (grad_params == nullptr) return 0;
     sss_unpack_grad_kernel<<<2 * p->nb_states, 128, 0, st>>>(p->stages, 2 * p->nb_states, p->rows_pad, p->k_pad, workspace, grad_params);
     SN_CHECK_LAUNCH("sss_unpack_grad_kernel");
     return 0;

@@ -3708,9 +3708,11 @@ int sn_sss_tc_backward(const sn_sss_tc_plan* p, const float* params, const float
                        int64_t ldgy, const float* states, float* workspace, float* grad_params, float* grad_bias, float* grad_x, int64_t ldgx,
                        int64_t B, sn_stream_t stream) {
     if (int rc = check_tc_plan(p)) return rc;
-    SN_CHECK_ARG(params && coef && x && grad_y && states && workspace && grad_params, "sss_tc_backward: NULL buffer");
+    SN_CHECK_ARG(params && coef && x && grad_y && states && workspace, "sss_tc_backward: NULL buffer");
+    SN_CHECK_ARG(grad_params != nullptr || grad_x != nullptr, "sss_tc_backward: grad_params and grad_x are both NULL (nothing to compute)");
     SN_CHECK_ARG(ldx >= p->input_dim && ldgy >= p->output_dim, "sss_tc_backward: leading dimension too small");
     SN_CHECK_ARG((ldgy & 3) == 0 && (reinterpret_cast<uintptr_t>(grad_y) & 15) == 0, "sss_tc_backward: grad_y must be 16-byte aligned with a row pitch multiple of 4");
+    SN_CHECK_ARG(grad_x == nullptr || ldgx >= p->input_dim, "sss_tc_backward: grad_x leading dimension too small");
     if (B <= 0) return 0;
     cudaStream_t st = snb::as_stream(stream);
     const float* SC = coef + (size_t)p->nchunks * WROWS * WCOLS;
@@ -3764,7 +3766,6 @@ int sn_sss_tc_backward(const sn_sss_tc_plan* p, const float* params, const float
     if (grad_x != nullptr) {
         // grad_u_j = [gy_j | lambda_{j+1} | mu_j] W_j  (W_j = [T_j ; R_j ; R'_j], 64 x 160): two small tensor-core GEMMs per chunk on the
         // adjoints the scans just left in L.  Optional path (the reference training loop never asks for it, training_helpers.py:34).
-        SN_CHECK_ARG(ldgx >= p->input_dim, "sss_tc_backward: grad_x leading dimension too small");
         float* Wsum = scratch + (size_t)p->nchunks * 2 * BB_SCR;
         SN_LAUNCH("sss_tc_wsum_kernel", st, sss_tc_wsum_kernel<<<p->nchunks, 256, 0, st>>>(coef, Wsum));
         std::vector<sn_sss_tc_chunk> hc(p->nchunks);
@@ -3777,6 +3778,11 @@ int sn_sss_tc_backward(const sn_sss_tc_plan* p, const float* params, const float
             if (int rc = snb::gemm_f32(false, false, (int)B, hc[j].ncols, kout, 1.f, grad_y + hc[j].row0, ldgy, Wj, WCOLS, 0.f, gxj, ldgx, nullptr, st)) return rc;
             if (int rc = snb::gemm_f32(false, false, (int)B, hc[j].ncols, 32, 1.f, L + (size_t)j * B * 32, 32, Wj + (size_t)PO * WCOLS, WCOLS, 1.f, gxj, ldgx, nullptr, st, true)) return rc;
         }
+    }
+    if (grad_params == nullptr) {   // input gradient only (frozen parameters): no gradient GEMM, no build backward
+        if (bias_later)
+            if (int rc = snb::colsum_accumulate(grad_y, ldgy, B, p->output_dim, grad_bias, st)) return rc;
+        return 0;
     }
     SN_CHECK_CUDA(cudaMemsetAsync(dM, 0, (size_t)p->nchunks * 64 * DMC * sizeof(float), st));
     CUtensorMap mx, mg, ml, ms;

@@ -100,17 +100,21 @@ def _check_params_unchanged(ctx, layer):
 
 class _SSSFunction(torch.autograd.Function):
     """fwd: sn_sss_forward (saves chunk-entry state checkpoints); bwd: sn_sss_backward accumulating
-    straight into the layer's flat gradient buffer (every ``p.grad`` is a view of it)."""
+    straight into the layer's flat gradient buffer (every ``p.grad`` is a view of it) and / or returning
+    the gradient w.r.t. the input features.
+
+    ``anchor`` is passed (a leaf that requires grad) when the parameters take gradients; ``save`` when a
+    backward can run at all (parameters or ``U`` need a gradient).  Grad mode is always off inside
+    Function.forward, so the layer decides both."""
 
     @staticmethod
-    def forward(ctx, U, anchor, layer):
+    def forward(ctx, U, anchor, layer, save):
         B = U.shape[0]
         plan = layer._device_plan(U.device)
         packed = layer._packed_params(plan)
         y = torch.empty((B, layer.output_dim), dtype=torch.float32, device=U.device)
-        need_grad = anchor is not None   # (grad mode is always off inside Function.forward)
         ckpt = None
-        if need_grad:
+        if save:
             nck = _lib.lib().sn_sss_ckpt_floats(ctypes.byref(plan["struct"]), B)
             ckpt = torch.empty(max(int(nck), 1), dtype=torch.float32, device=U.device)
         bias = layer.bias if layer.use_bias else None
@@ -119,6 +123,7 @@ class _SSSFunction(torch.autograd.Function):
         _lib.check(rc, "sn_sss_forward")
         ctx.layer = layer
         ctx.plan = plan
+        ctx.param_grad = anchor is not None
         ctx.param_version = _param_version(layer)
         ctx.save_for_backward(U, ckpt, packed)
         return y
@@ -128,27 +133,25 @@ class _SSSFunction(torch.autograd.Function):
         layer, plan = ctx.layer, ctx.plan
         _check_params_unchanged(ctx, layer)
         U, ckpt, packed = ctx.saved_tensors
-        if ctx.needs_input_grad[0]:
-            raise RuntimeError("SSSLayer: the SIMT kernels (layers outside the tensor-core path's limits) do not return the gradient "
-                               "w.r.t. the input features; the tensor-core path does")
+        grad_x = torch.empty_like(U) if ctx.needs_input_grad[0] else None
         grad_y = grad_y.contiguous()
         if grad_y.dtype != torch.float32:
             grad_y = grad_y.float()
-        g = layer._prepare_grad_accumulation()
-        gbias = g[:layer.output_dim] if (layer.use_bias and layer.bias.requires_grad) else None
-        ws = layer._backward_workspace(plan)
+        g = layer._prepare_grad_accumulation() if ctx.param_grad else None
+        gbias = g[:layer.output_dim] if (g is not None and layer.use_bias and layer.bias.requires_grad) else None
+        ws = layer._backward_workspace(plan) if g is not None else None
         rc = _lib.lib().sn_sss_backward(ctypes.byref(plan["struct"]), _lib.ptr(packed), _lib.ptr(U), U.stride(0),
                                         _lib.ptr(grad_y), grad_y.stride(0), _lib.ptr(ckpt), _lib.ptr(ws), _lib.ptr(g), _lib.ptr(gbias),
-                                        None, 0, U.shape[0], _lib.stream_ptr())
+                                        _lib.ptr(grad_x), grad_x.stride(0) if grad_x is not None else 0, U.shape[0], _lib.stream_ptr())
         _lib.check(rc, "sn_sss_backward")
-        return None, None, None
+        return grad_x, None, None, None
 
 
 class _SSSTCFunction(torch.autograd.Function):
-    """Tensor-core path (csrc/sss_tc.cu): sn_sss_tc_build + sn_sss_tc_forward, sn_sss_tc_backward."""
+    """Tensor-core path (csrc/sss_tc.cu): sn_sss_tc_build + sn_sss_tc_forward, sn_sss_tc_backward.  Arguments as _SSSFunction."""
 
     @staticmethod
-    def forward(ctx, U, anchor, layer):
+    def forward(ctx, U, anchor, layer, save):
         B = U.shape[0]
         L = _lib.lib()
         tc = layer._tc_plan(U.device)
@@ -166,8 +169,9 @@ class _SSSTCFunction(torch.autograd.Function):
         _lib.check(rc, "sn_sss_tc_forward")
         ctx.layer = layer
         ctx.tc = tc
+        ctx.param_grad = anchor is not None
         ctx.param_version = _param_version(layer)
-        if anchor is not None:
+        if save:
             ctx.save_for_backward(U, states)
         return y
 
@@ -183,15 +187,15 @@ class _SSSTCFunction(torch.autograd.Function):
         L = _lib.lib()
         ps = ctypes.byref(tc["struct"])
         B = U.shape[0]
-        g = layer._prepare_grad_accumulation()
-        gbias = g[:layer.output_dim] if (layer.use_bias and layer.bias.requires_grad) else None
+        g = layer._prepare_grad_accumulation() if ctx.param_grad else None
+        gbias = g[:layer.output_dim] if (g is not None and layer.use_bias and layer.bias.requires_grad) else None
         ws = torch.empty(max(int(L.sn_sss_tc_backward_workspace_floats(ps, B)), 1), dtype=torch.float32, device=U.device)
         # tc["coef"] still holds the chunk matrices of the forward (rebuilt at every forward from the flat parameters)
         rc = L.sn_sss_tc_backward(ps, _lib.ptr(layer.__dict__["_flat"]), _lib.ptr(tc["coef"]), _lib.ptr(U), U.stride(0),
                                   _lib.ptr(grad_y), grad_y.stride(0), _lib.ptr(states), _lib.ptr(ws), _lib.ptr(g), _lib.ptr(gbias),
                                   _lib.ptr(grad_x), grad_x.stride(0) if grad_x is not None else 0, B, _lib.stream_ptr())
         _lib.check(rc, "sn_sss_tc_backward")
-        return grad_x, None, None
+        return grad_x, None, None, None
 
 
 class SSSLayer(FlatParamsMixin, StructuredLayer):
@@ -465,9 +469,11 @@ class SSSLayer(FlatParamsMixin, StructuredLayer):
             if anchor is None or anchor.device != U.device:
                 anchor = torch.zeros(1, device=U.device, requires_grad=True)
                 self.__dict__["_dev_anchor"] = anchor
-            any_grad = torch.is_grad_enabled() and any(p.requires_grad for p in (self.A[0], self.D[0]))
+            # the first parameter (the bias, or A[0]) decides at once for a trainable layer; a frozen one is walked in full
+            param_grad = torch.is_grad_enabled() and any(p.requires_grad for p in self._flat_param_list())
+            save = param_grad or (torch.is_grad_enabled() and U.requires_grad)
             fn = _SSSTCFunction if self._use_tc_path() else _SSSFunction
-            return fn.apply(U, anchor if any_grad else None, self)
+            return fn.apply(U, anchor if param_grad else None, self, save)
         else:
             # the budget admits not even a block-diagonal D: reference returns zeros (sss_layer.py:130-131)
             return torch.zeros((U.shape[0], self.output_dim), device=U.device)
