@@ -165,26 +165,34 @@ int sn_lr_backward_f32(const float* x, int64_t ldx, const float* grad_y, int64_t
 /* Low-rank layer, bf16 tensor-core path (tcgen05 / TMEM / TMA; BASELINE config C2).  All bf16 matrices are row-major
  * with 16-byte aligned rows (row pitch multiple of 8 elements).  sn_lr_tc_cast_params makes the bf16 copies
  * L (out x rank), L^T (rank x lt_ld) and R (rank x in) of the fp32 master parameters.  Backward scratch (bf16):
- * ghid (B x rank), gyt (out x ldt), ht (rank x ldt), ght (rank x ldt), xt (in x ldt), ldt = B rounded up to 8;
- * grad_left / grad_right / grad_bias are fp32 and accumulated. */
+ * ghid (B x rank); gyt (out x ldt) and ht (rank x ldt), needed only with grad_left; ght (rank x ldt) and xt (in x ldt), needed
+ * only with grad_right; ldt = B rounded up to 8;
+ * grad_left / grad_right / grad_bias are fp32, accumulated, and each may be NULL.  grad_x (nullable, bf16, B x in, row
+ * pitch ldgx >= in_dim and a multiple of 8) = ghid R, written, bitwise reproducible (no split-K); it needs right_bf16 (the
+ * R of sn_lr_tc_cast_params) and right_t, scratch for R^T (in x rank); both may be NULL when grad_x is. */
 int sn_lr_tc_cast_params(const float* left, const float* right, void* left_bf16, void* left_t_bf16, int64_t lt_ld, void* right_bf16,
                          int in_dim, int out_dim, int rank, sn_stream_t stream);
 int sn_lr_tc_forward(const void* x, int64_t ldx, const void* left_bf16, const void* right_bf16, const float* bias, void* hidden, void* y,
                      int64_t ldy, int64_t B, int in_dim, int out_dim, int rank, sn_stream_t stream);
-int sn_lr_tc_backward(const void* x, int64_t ldx, const void* grad_y, int64_t ldgy, const void* left_t_bf16, int64_t lt_ld, const void* hidden,
-                      void* ghid, void* gyt, void* ht, void* ght, void* xt, int64_t ldt, float* grad_left, float* grad_right, float* grad_bias,
-                      int64_t B, int in_dim, int out_dim, int rank, sn_stream_t stream);
+int sn_lr_tc_backward(const void* x, int64_t ldx, const void* grad_y, int64_t ldgy, const void* left_t_bf16, int64_t lt_ld,
+                      const void* right_bf16, const void* hidden, void* ghid, void* gyt, void* ht, void* ght, void* xt, int64_t ldt,
+                      void* right_t, float* grad_left, float* grad_right, float* grad_bias, void* grad_x, int64_t ldgx, int64_t B,
+                      int in_dim, int out_dim, int rank, sn_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
  * H-matrix layer -- replaces HMatLayer.forward (layers/hmat_layer.py:34-49) and its backward.
  *   leaves: device table, 8 int32 per leaf {row_start, rows, col_start, cols, rank, off_left, off_right, 0};
  *   params: flat buffer holding left_lr (rows x rank) / right_lr (rank x cols) of every leaf at those offsets;
- *   grad_params has the same layout.
+ *   grad_params has the same layout (accumulated).  sn_hmat_backward: grad_x (nullable; row pitch ldgx >= in_dim) = grad_y W,
+ *   written; its leaves add through shared-memory atomics, so it agrees with other summation orders to rounding, not bitwise.
+ *   grad_params may be NULL when grad_x is not (input gradient only: the leaf-gradient kernel does not run; grad_bias is still
+ *   accumulated when given).  Both NULL is an error.
  * ------------------------------------------------------------------------------------------ */
 int sn_hmat_forward(const int32_t* leaves, int nleaves, const float* params, const float* x, int64_t ldx, float* y, int64_t ldy,
                     const float* bias, int64_t B, int in_dim, int out_dim, sn_stream_t stream);
 int sn_hmat_backward(const int32_t* leaves, int nleaves, const float* params, const float* x, int64_t ldx, const float* grad_y,
-                     int64_t ldgy, float* grad_params, float* grad_bias, int64_t B, int in_dim, int out_dim, sn_stream_t stream);
+                     int64_t ldgy, float* grad_params, float* grad_bias, float* grad_x, int64_t ldgx, int64_t B, int in_dim, int out_dim,
+                     sn_stream_t stream);
 /* Dense-block path (default for layers whose dense matrix fits): W = the H-matrix as a dense (out_dim x in_dim) matrix built from
  * the leaves (max_rows = the tallest leaf), applied / differentiated with sn_dense_apply / sn_dense_weight_grad on the tensor cores,
  * and the dense gradient projected back onto the leaf factors (accumulated into grad_params). */
@@ -217,12 +225,17 @@ typedef struct sn_psm_factor {
     float *val_fwd, *val_tr, *grad_packed;
 } sn_psm_factor;
 /* acts (nullable): sn_psm_acts_floats floats; the forward keeps the input of every factor but the last there ([B][cols_k] row-major,
- * factor 0 first) and the backward reads them instead of recomputing them from x */
+ * factor 0 first) and the backward reads them instead of recomputing them from x.
+ * sn_psm_backward: grad_x (nullable; row pitch ldgx >= in_dim) = grad_y S_0 .. S_{n-1}, written, bitwise reproducible.  The factor
+ * gradient buffers (grad_vals, grad_packed of every factor) are all set or all NULL; all NULL is allowed only when grad_x is set
+ * (input gradient only, e.g. frozen factors: the forward kernel runs on the transposed chain and acts is not read; grad_bias is
+ * still accumulated when given).  val_tr is needed in both modes. */
 size_t sn_psm_acts_floats(const sn_psm_factor* factors_host, int nf, int64_t B);
 int sn_psm_forward(const sn_psm_factor* factors_host, int nf, const float* x, int64_t ldx, float* y, int64_t ldy, const float* bias,
                    float* acts, int64_t B, int in_dim, int out_dim, sn_stream_t stream);
 int sn_psm_backward(const sn_psm_factor* factors_host, int nf, const float* x, int64_t ldx, const float* grad_y, int64_t ldgy,
-                    const float* acts, float* grad_bias, int64_t B, int in_dim, int out_dim, sn_stream_t stream);
+                    const float* acts, float* grad_bias, float* grad_x, int64_t ldgx, int64_t B, int in_dim, int out_dim,
+                    sn_stream_t stream);
 
 /* Dense-product path of the PSM layer for large batches (csrc/psm.cu): the batch-independent product W = S_0 .. S_{n-1} is
  * multiplied out once per call (transposed prefix products, kept in `prefix` for the backward), applied / differentiated on the

@@ -97,7 +97,7 @@ def _declare(lib):
     lib.sn_hmat_forward.restype = c_int
     lib.sn_hmat_forward.argtypes = [vp, i32, vp, vp, i64, vp, i64, vp, i64, i32, i32, vp]
     lib.sn_hmat_backward.restype = c_int
-    lib.sn_hmat_backward.argtypes = [vp, i32, vp, vp, i64, vp, i64, vp, vp, i64, i32, i32, vp]
+    lib.sn_hmat_backward.argtypes = [vp, i32, vp, vp, i64, vp, i64, vp, vp, vp, i64, i64, i32, i32, vp]
     lib.sn_hmat_build_dense.restype = c_int
     lib.sn_hmat_build_dense.argtypes = [vp, i32, i32, vp, i32, vp, vp, i32, i32, vp]
     lib.sn_hmat_project_grad.restype = c_int
@@ -106,7 +106,7 @@ def _declare(lib):
     lib.sn_psm_forward.restype = c_int
     lib.sn_psm_forward.argtypes = [PF, i32, vp, i64, vp, i64, vp, vp, i64, i32, i32, vp]
     lib.sn_psm_backward.restype = c_int
-    lib.sn_psm_backward.argtypes = [PF, i32, vp, i64, vp, i64, vp, vp, i64, i32, i32, vp]
+    lib.sn_psm_backward.argtypes = [PF, i32, vp, i64, vp, i64, vp, vp, vp, i64, i64, i32, i32, vp]
     lib.sn_psm_acts_floats.restype = c_size_t
     lib.sn_psm_acts_floats.argtypes = [PF, i32, i64]
     PD = POINTER(SnPsmDenseFactor)
@@ -154,7 +154,7 @@ def _declare(lib):
     lib.sn_lr_tc_forward.restype = c_int
     lib.sn_lr_tc_forward.argtypes = [vp, i64, vp, vp, vp, vp, vp, i64, i64, i32, i32, i32, vp]
     lib.sn_lr_tc_backward.restype = c_int
-    lib.sn_lr_tc_backward.argtypes = [vp, i64, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp, i64, vp, vp, vp, i64, i32, i32, i32, vp]
+    lib.sn_lr_tc_backward.argtypes = [vp, i64, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp, vp, i64, vp, vp, vp, vp, vp, i64, i64, i32, i32, i32, vp]
     f32 = ctypes.c_float
     lib.sn_ce_loss.restype = c_int
     lib.sn_ce_loss.argtypes = [vp, i64, vp, i64, i32, vp, vp, vp, i64, vp]

@@ -46,21 +46,40 @@ __device__ __forceinline__ void stage1(const Leaf& lf, const float* __restrict__
     }
 }
 
+// the transposed stage 1 (as in hmat_bwd_kernel): gt[kk][s] = sum_r L_c[r][kc+kk] * gy[r0+r][s]
 template <int NS>
+__device__ __forceinline__ void stage1_tr(const Leaf& lf, const float* __restrict__ L, int kc, int kn, const float* gs, float* gtb,
+                                          int s, int h) {
+    constexpr int H = 32 / NS;
+    for (int kk = h; kk < kn; kk += H) {
+        const float* gv = gs + (size_t)lf.r0 * NS + s;
+        float acc = 0.f;
+#pragma unroll 4
+        for (int r = 0; r < lf.rows; ++r) acc = fmaf(__ldg(L + (size_t)r * lf.k + kc + kk), gv[r * NS], acc);
+        gtb[kk * NS + s] = acc;
+    }
+}
+
+// TR = false: y = forward(x) + bias.  TR = true: every leaf transposed, y = grad_x (B x in_dim) from x = grad_y (B x out_dim):
+//     stage 1  t[kk][s]      = sum_r L_c[r][kk] * gy[r0+r][s]
+//     stage 2  gx[c0+col][s] += sum_kk R_c[kk][col] * t[kk][s]
+// with the forward's shared-memory layout and size (an input tile and an output tile of in_dim + out_dim features in all); bias unused.
+template <int NS, bool TR>
 __global__ void __launch_bounds__(HM_THREADS)
 hmat_fwd_kernel(const Leaf* __restrict__ leaves, int nleaves, const float* __restrict__ params, const float* __restrict__ x,
                 long ldx, float* __restrict__ y, long ldy, const float* __restrict__ bias, long B, int in_dim, int out_dim) {
     extern __shared__ __align__(16) float smem[];
+    const int nx = TR ? out_dim : in_dim, ny = TR ? in_dim : out_dim;
     float* xs = smem;
-    float* ys = xs + (size_t)in_dim * NS;
-    float* tb = ys + (size_t)out_dim * NS + (threadIdx.x >> 5) * (HM_KCHUNK * NS);
+    float* ys = xs + (size_t)nx * NS;
+    float* tb = ys + (size_t)ny * NS + (threadIdx.x >> 5) * (HM_KCHUNK * NS);
     const long t0 = (long)blockIdx.x * NS;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int s = lane % NS, h = lane / NS;
     constexpr int H = 32 / NS;
 
-    load_tile<NS>(x, ldx, t0, B, in_dim, xs);
-    for (int e = threadIdx.x; e < out_dim * NS; e += HM_THREADS) ys[e] = bias ? __ldg(bias + e / NS) : 0.f;
+    load_tile<NS>(x, ldx, t0, B, nx, xs);
+    for (int e = threadIdx.x; e < ny * NS; e += HM_THREADS) ys[e] = (!TR && bias) ? __ldg(bias + e / NS) : 0.f;
     __syncthreads();
 
     for (int c = warp; c < nleaves; c += HM_WARPS) {
@@ -69,13 +88,25 @@ hmat_fwd_kernel(const Leaf* __restrict__ leaves, int nleaves, const float* __res
         const float* R = params + lf.offR;
         for (int kc = 0; kc < lf.k; kc += HM_KCHUNK) {
             const int kn = min(HM_KCHUNK, lf.k - kc);
-            stage1<NS>(lf, R, kc, kn, xs, tb, s, h);
+            if (TR) stage1_tr<NS>(lf, L, kc, kn, xs, tb, s, h);
+            else stage1<NS>(lf, R, kc, kn, xs, tb, s, h);
             __syncwarp();
-            for (int r = h; r < lf.rows; r += H) {
-                const float* Lrow = L + (size_t)r * lf.k + kc;
-                float acc = 0.f;
-                for (int kk = 0; kk < kn; ++kk) acc = fmaf(__ldg(Lrow + kk), tb[kk * NS + s], acc);
-                atomicAdd(&ys[(size_t)(lf.r0 + r) * NS + s], acc);
+            if (TR) {
+                for (int col = h; col < lf.cols; col += H) {
+                    const float* Rcol = R + (size_t)kc * lf.cols + col;
+                    float acc = 0.f;
+                    // left to the compiler, this loop costs the NS = 8 / 16 instantiations a 12-byte spill; "#pragma unroll 1" avoids it
+                    // but made the C4-H grad_x 0.83 ms (13 %) slower on a B200 (DESIGN.md 4.5)
+                    for (int kk = 0; kk < kn; ++kk) acc = fmaf(__ldg(Rcol + (size_t)kk * lf.cols), tb[kk * NS + s], acc);
+                    atomicAdd(&ys[(size_t)(lf.c0 + col) * NS + s], acc);
+                }
+            } else {
+                for (int r = h; r < lf.rows; r += H) {
+                    const float* Lrow = L + (size_t)r * lf.k + kc;
+                    float acc = 0.f;
+                    for (int kk = 0; kk < kn; ++kk) acc = fmaf(__ldg(Lrow + kk), tb[kk * NS + s], acc);
+                    atomicAdd(&ys[(size_t)(lf.r0 + r) * NS + s], acc);
+                }
             }
             __syncwarp();
         }
@@ -84,7 +115,7 @@ hmat_fwd_kernel(const Leaf* __restrict__ leaves, int nleaves, const float* __res
     for (int sidx = 0; sidx < NS; ++sidx) {
         if (t0 + sidx >= B) break;
         float* row = y + (size_t)(t0 + sidx) * ldy;
-        for (int o = threadIdx.x; o < out_dim; o += HM_THREADS) row[o] = ys[o * NS + sidx];
+        for (int o = threadIdx.x; o < ny; o += HM_THREADS) row[o] = ys[o * NS + sidx];
     }
 }
 
@@ -249,25 +280,17 @@ hmat_project_grad_kernel(const Leaf* __restrict__ leaves, const int2* __restrict
     }
 }
 
-}  // namespace
-
-extern "C" {
-
-// leaves: device table, 8 int32 per leaf {row_start, rows, col_start, cols, rank, off_left, off_right, 0};
-// params: flat parameter buffer holding left_lr (rows x k) and right_lr (k x cols) of every leaf at those offsets.
-int sn_hmat_forward(const int32_t* leaves, int nleaves, const float* params, const float* x, int64_t ldx, float* y, int64_t ldy,
-                    const float* bias, int64_t B, int in_dim, int out_dim, sn_stream_t stream) {
-    SN_CHECK_ARG(params && x && y && (leaves || nleaves == 0), "hmat_forward: NULL buffer");
-    if (B <= 0) return 0;
-    cudaStream_t st = snb::as_stream(stream);
-    const Leaf* lv = reinterpret_cast<const Leaf*>(leaves);
+// Launches hmat_fwd_kernel<NS, TR> at the largest sample tile NS whose shared memory fits: 0 = launched, -1 = fits at no NS.
+template <bool TR>
+int hm_launch_fwd(const Leaf* lv, int nleaves, const float* params, const float* x, long ldx, float* y, long ldy, const float* bias, long B,
+                  int in_dim, int out_dim, cudaStream_t st) {
 #define HM_LAUNCH_FWD(NS)                                                                                                  \
     {                                                                                                                      \
         size_t smem = hm_smem<NS>(in_dim, out_dim, false);                                                                 \
         if (smem <= 227 * 1024) {                                                                                          \
-            SN_SET_MAX_SMEM((int)smem, hmat_fwd_kernel<NS>); \
-            hmat_fwd_kernel<NS><<<(unsigned)((B + NS - 1) / NS), HM_THREADS, smem, st>>>(lv, nleaves, params, x, ldx, y, ldy, bias, B, in_dim, out_dim); \
-            SN_CHECK_LAUNCH("hmat_fwd_kernel");                                                                            \
+            SN_SET_MAX_SMEM((int)smem, hmat_fwd_kernel<NS, TR>); \
+            hmat_fwd_kernel<NS, TR><<<(unsigned)((B + NS - 1) / NS), HM_THREADS, smem, st>>>(lv, nleaves, params, x, ldx, y, ldy, bias, B, in_dim, out_dim); \
+            SN_CHECK_LAUNCH(TR ? "hmat_fwd_kernel<TR>" : "hmat_fwd_kernel");                                               \
             return 0;                                                                                                      \
         }                                                                                                                  \
     }
@@ -276,18 +299,12 @@ int sn_hmat_forward(const int32_t* leaves, int nleaves, const float* params, con
     HM_LAUNCH_FWD(4)
     HM_LAUNCH_FWD(2)
 #undef HM_LAUNCH_FWD
-    snb::set_error("hmat_forward: in_dim + out_dim = %d does not fit in shared memory", in_dim + out_dim);
-    return 1;
+    return -1;
 }
 
-int sn_hmat_backward(const int32_t* leaves, int nleaves, const float* params, const float* x, int64_t ldx, const float* grad_y,
-                     int64_t ldgy, float* grad_params, float* grad_bias, int64_t B, int in_dim, int out_dim, sn_stream_t stream) {
-    SN_CHECK_ARG(params && x && grad_y && grad_params && (leaves || nleaves == 0), "hmat_backward: NULL buffer");
-    if (B <= 0) return 0;
-    cudaStream_t st = snb::as_stream(stream);
-    const Leaf* lv = reinterpret_cast<const Leaf*>(leaves);
-    if (grad_bias)
-        if (int rc = snb::colsum_accumulate(grad_y, ldgy, B, out_dim, grad_bias, st)) return rc;
+// Launches hmat_bwd_kernel<NS> as above: 0 = launched, -1 = fits at no NS.
+int hm_launch_bwd(const Leaf* lv, int nleaves, const float* params, const float* x, long ldx, const float* grad_y, long ldgy, float* grad_params,
+                  long B, int in_dim, int out_dim, cudaStream_t st) {
 #define HM_LAUNCH_BWD(NS)                                                                                                  \
     {                                                                                                                      \
         size_t smem = hm_smem<NS>(in_dim, out_dim, true);                                                                  \
@@ -303,8 +320,59 @@ int sn_hmat_backward(const int32_t* leaves, int nleaves, const float* params, co
     HM_LAUNCH_BWD(4)
     HM_LAUNCH_BWD(2)
 #undef HM_LAUNCH_BWD
-    snb::set_error("hmat_backward: in_dim + out_dim = %d does not fit in shared memory", in_dim + out_dim);
-    return 1;
+    return -1;
+}
+
+}  // namespace
+
+extern "C" {
+
+// leaves: device table, 8 int32 per leaf {row_start, rows, col_start, cols, rank, off_left, off_right, 0};
+// params: flat parameter buffer holding left_lr (rows x k) and right_lr (k x cols) of every leaf at those offsets.
+int sn_hmat_forward(const int32_t* leaves, int nleaves, const float* params, const float* x, int64_t ldx, float* y, int64_t ldy,
+                    const float* bias, int64_t B, int in_dim, int out_dim, sn_stream_t stream) {
+    SN_CHECK_ARG(params && x && y && (leaves || nleaves == 0), "hmat_forward: NULL buffer");
+    if (B <= 0) return 0;
+    const int rc = hm_launch_fwd<false>(reinterpret_cast<const Leaf*>(leaves), nleaves, params, x, ldx, y, ldy, bias, B, in_dim, out_dim,
+                                        snb::as_stream(stream));
+    if (rc < 0) {
+        snb::set_error("hmat_forward: in_dim + out_dim = %d does not fit in shared memory", in_dim + out_dim);
+        return 1;
+    }
+    return rc;
+}
+
+// grad_params (nullable when grad_x is not) += the leaf gradients; grad_x (nullable; row pitch ldgx >= in_dim) = grad_y W, written by
+// a second launch: the forward kernel with every leaf transposed, so every layer whose forward runs also gets its grad_x.
+int sn_hmat_backward(const int32_t* leaves, int nleaves, const float* params, const float* x, int64_t ldx, const float* grad_y,
+                     int64_t ldgy, float* grad_params, float* grad_bias, float* grad_x, int64_t ldgx, int64_t B, int in_dim, int out_dim,
+                     sn_stream_t stream) {
+    SN_CHECK_ARG(params && x && grad_y && (leaves || nleaves == 0), "hmat_backward: NULL buffer");
+    SN_CHECK_ARG(grad_params || grad_x, "hmat_backward: grad_params and grad_x are both NULL");
+    SN_CHECK_ARG(grad_x == nullptr || ldgx >= in_dim, "hmat_backward: grad_x leading dimension too small (ldgx %lld < in_dim %d)",
+                 (long long)ldgx, in_dim);
+    if (B <= 0) return 0;
+    cudaStream_t st = snb::as_stream(stream);
+    const Leaf* lv = reinterpret_cast<const Leaf*>(leaves);
+    if (grad_bias)
+        if (int rc = snb::colsum_accumulate(grad_y, ldgy, B, out_dim, grad_bias, st)) return rc;
+    if (grad_params) {
+        const int rc = hm_launch_bwd(lv, nleaves, params, x, ldx, grad_y, ldgy, grad_params, B, in_dim, out_dim, st);
+        if (rc < 0) {
+            snb::set_error("hmat_backward: in_dim + out_dim = %d does not fit in shared memory", in_dim + out_dim);
+            return 1;
+        }
+        if (rc) return rc;
+    }
+    if (grad_x) {
+        const int rc = hm_launch_fwd<true>(lv, nleaves, params, grad_y, ldgy, grad_x, ldgx, nullptr, B, in_dim, out_dim, st);
+        if (rc < 0) {
+            snb::set_error("hmat_backward: in_dim + out_dim = %d does not fit in shared memory", in_dim + out_dim);
+            return 1;
+        }
+        if (rc) return rc;
+    }
+    return 0;
 }
 
 // W[out_dim x in_dim] (row-major, dense) = the H-matrix (zero where no leaf with rank > 0 lives)

@@ -279,12 +279,19 @@ int sn_lr_tc_forward(const void* x, int64_t ldx, const void* left_bf16, const vo
 }
 
 // grad_left (out x rank), grad_right (rank x in), grad_bias (out) are fp32 and accumulated.  Scratch (bf16): ghid (B x rank),
-// gyt (out x ldt), ht (rank x ldt), ght (rank x ldt), xt (in x ldt) with ldt = B rounded up to a multiple of 8.
-int sn_lr_tc_backward(const void* x, int64_t ldx, const void* grad_y, int64_t ldgy, const void* left_t_bf16, int64_t lt_ld, const void* hidden,
-                      void* ghid, void* gyt, void* ht, void* ght, void* xt, int64_t ldt, float* grad_left, float* grad_right, float* grad_bias,
-                      int64_t B, int in_dim, int out_dim, int rank, sn_stream_t stream) {
-    SN_CHECK_ARG(x && grad_y && left_t_bf16 && hidden && ghid && gyt && ht && ght && xt, "lr_tc_backward: NULL buffer");
+// gyt (out x ldt) and ht (rank x ldt) when grad_left is given, ght (rank x ldt) and xt (in x ldt) when grad_right is, with ldt = B rounded
+// up to a multiple of 8; right_t (in x rank) when grad_x (bf16, B x in, written) is asked for.
+int sn_lr_tc_backward(const void* x, int64_t ldx, const void* grad_y, int64_t ldgy, const void* left_t_bf16, int64_t lt_ld,
+                      const void* right_bf16, const void* hidden, void* ghid, void* gyt, void* ht, void* ght, void* xt, int64_t ldt,
+                      void* right_t, float* grad_left, float* grad_right, float* grad_bias, void* grad_x, int64_t ldgx, int64_t B,
+                      int in_dim, int out_dim, int rank, sn_stream_t stream) {
+    SN_CHECK_ARG(x && grad_y && left_t_bf16 && hidden && ghid, "lr_tc_backward: NULL buffer");
+    SN_CHECK_ARG((grad_left == nullptr || (gyt && ht)) && (grad_right == nullptr || (ght && xt)), "lr_tc_backward: NULL transpose scratch");
     SN_CHECK_ARG(ldt >= B && ldt % 8 == 0, "lr_tc_backward: ldt must be B rounded up to a multiple of 8");
+    SN_CHECK_ARG(grad_x == nullptr || (right_bf16 && right_t), "lr_tc_backward: grad_x needs right_bf16 and the right_t scratch");
+    SN_CHECK_ARG(grad_x == nullptr || ldgx >= in_dim, "lr_tc_backward: grad_x leading dimension too small (ldgx %lld < in_dim %d)",
+                 (long long)ldgx, in_dim);
+    SN_CHECK_ARG(grad_x == nullptr || ldgx % 8 == 0, "lr_tc_backward: grad_x leading dimension %lld is not a multiple of 8", (long long)ldgx);
     if (B <= 0) return 0;
     cudaStream_t st = snb::as_stream(stream);
     using namespace snb::tc;
@@ -302,6 +309,10 @@ int sn_lr_tc_backward(const void* x, int64_t ldx, const void* grad_y, int64_t ld
     }
     // gh = gy L : A = gy (B x out), B operand = L^T (rank x out), K = out
     if (int rc = gemm_bf16_tc<64, STORE_BF16>((int)B, rank, out_dim, grad_y, ldgy, left_t_bf16, lt_ld, ghid, rank, nullptr, 1.f, 1, st)) return rc;
+    if (grad_x) {   // grad_x = gh R : B operand = R^T (in x rank, K-major); no split-K, so every element has one owner
+        if (int rc = transpose_bf16((const bf16*)right_bf16, in_dim, (bf16*)right_t, rank, rank, in_dim, st)) return rc;
+        if (int rc = gemm_bf16_tc<128, STORE_BF16>((int)B, in_dim, rank, ghid, rank, right_t, rank, grad_x, ldgx, nullptr, 1.f, 1, st)) return rc;
+    }
     if (grad_bias) {
         dim3 grid(snb::ceil_div(out_dim, 256), (unsigned)((B + 63) / 64));
         SN_LAUNCH("colsum_bf16_kernel", s2, colsum_bf16_kernel<<<grid, 128, 0, s2>>>((const bf16*)grad_y, ldgy, B, out_dim, grad_bias));

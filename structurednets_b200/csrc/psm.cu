@@ -161,9 +161,13 @@ psm_fwd_kernel(Chain ch, const float* __restrict__ x, long ldx, float* __restric
 }
 
 // Backward with the activations the forward kept: two buffers.  G holds the gradient entering factor k from the output side, P the
-// input of factor k; after dS_k the product S_k^T G overwrites P and becomes the next G.
+// input of factor k; after dS_k the product S_k^T G overwrites P and becomes the next G.  gx (nullable): after the last factor's dS,
+// one more S_{n-1}^T G gives the tile's grad_x = gy S_0 .. S_{n-1}; each CTA writes only its own samples.  GX = (gx != nullptr): the
+// instantiation without grad_x is the kernel as it was before grad_x existed.
+template <bool GX>
 __global__ void __launch_bounds__(PSM_THREADS)
-psm_bwd_acts_kernel(Chain ch, const float* __restrict__ x, long ldx, const float* __restrict__ gy, long ldgy, long B, const float* __restrict__ acts) {
+psm_bwd_acts_kernel(Chain ch, const float* __restrict__ x, long ldx, const float* __restrict__ gy, long ldgy, long B, const float* __restrict__ acts,
+                    float* __restrict__ gx, long ldgx) {
     extern __shared__ __align__(16) float smem[];
     const size_t vec = (size_t)ch.maxdim * NS;
     float* G = smem;
@@ -177,19 +181,23 @@ psm_bwd_acts_kernel(Chain ch, const float* __restrict__ x, long ldx, const float
         off += (size_t)B * ch.f[k].cols;
         __syncthreads();
         dvals_ell(ch.f[k].fwd, G, P, ch.f[k].gpacked);
-        if (k + 1 < ch.nf) {
+        if (k + 1 < ch.nf || GX) {
             __syncthreads();                      // every warp is done reading P
             spmm_ell(ch.f[k].tr, G, P);           // S_k^T G
             __syncthreads();
             float* t = G; G = P; P = t;
         }
     }
+    if (GX) store_tile(gx, ldgx, t0, B, ch.in_dim, G);
 }
 
 // Three buffers: P / Q recompute the input of factor k from x (ping-pong), G holds the gradient that enters factor k from the
-// output side; S_k^T G lands in whichever of P / Q is free and becomes the next G.
+// output side; S_k^T G lands in whichever of P / Q is free and becomes the next G.  gx (nullable): as in psm_bwd_acts_kernel.
+// PSMLayer reaches GX = true only with one factor (with more, its forward keeps the activations whenever a factor takes a gradient);
+// sn_psm_backward callers that pass no acts reach it with any number of factors.
+template <bool GX>
 __global__ void __launch_bounds__(PSM_THREADS)
-psm_bwd_kernel(Chain ch, const float* __restrict__ x, long ldx, const float* __restrict__ gy, long ldgy, long B) {
+psm_bwd_kernel(Chain ch, const float* __restrict__ x, long ldx, const float* __restrict__ gy, long ldgy, long B, float* __restrict__ gx, long ldgx) {
     extern __shared__ __align__(16) float smem[];
     const size_t vec = (size_t)ch.maxdim * NS;
     float* P = smem;
@@ -207,17 +215,30 @@ psm_bwd_kernel(Chain ch, const float* __restrict__ x, long ldx, const float* __r
             float* t = P; P = Q; Q = t;
         }
         dvals_ell(ch.f[k].fwd, G, P, ch.f[k].gpacked);
-        if (k + 1 < ch.nf) {
+        if (k + 1 < ch.nf || GX) {
             spmm_ell(ch.f[k].tr, G, Q);   // S_k^T G (Q is free: the recomputed input sits in P)
             __syncthreads();
             float* t = G; G = Q; Q = t;
         }
     }
+    if (GX) store_tile(gx, ldgx, t0, B, ch.in_dim, G);
 }
 
-int make_chain(const sn_psm_factor* f, int nf, int in_dim, int out_dim, bool backward, Chain* ch) {
+// Raises psm_fwd_kernel's dynamic shared-memory limit.  The forward and the input-gradient-only backward both launch that kernel, and
+// SN_SET_MAX_SMEM remembers per call site what it set: a second site could lower the limit below what the first one believes it set.
+int fwd_kernel_smem(size_t smem) {
+    SN_SET_MAX_SMEM((int)smem, psm_fwd_kernel);
+    return 0;
+}
+
+// backward: the transposed patterns are needed, and the factor gradient buffers (grad_vals, grad_packed) are all set or all NULL;
+// *param_grad (backward only) tells which
+int make_chain(const sn_psm_factor* f, int nf, int in_dim, int out_dim, bool backward, Chain* ch, bool* param_grad = nullptr) {
     SN_CHECK_ARG(f != nullptr && nf >= 1 && nf <= PSM_MAX_FACTORS, "psm: need 1..%d factors", PSM_MAX_FACTORS);
     ch->nf = nf; ch->in_dim = in_dim; ch->out_dim = out_dim; ch->maxdim = in_dim > out_dim ? in_dim : out_dim;
+    bool any_grad = false;
+    for (int k = 0; k < nf; ++k) any_grad |= f[k].grad_vals != nullptr || f[k].grad_packed != nullptr;
+    if (param_grad != nullptr) *param_grad = any_grad;
     for (int k = 0; k < nf; ++k) {
         const sn_psm_factor& s = f[k];
         SN_CHECK_ARG(s.rows > 0 && s.cols > 0 && s.rows <= 65535 && s.cols <= 65535, "psm: factor %d is %d x %d (dimensions must be in 1..65535)", k, s.rows, s.cols);
@@ -231,7 +252,8 @@ int make_chain(const sn_psm_factor* f, int nf, int in_dim, int out_dim, bool bac
         F.gpacked = s.grad_packed;
         if (backward) {
             SN_CHECK_ARG(s.tr.rowmap && s.tr.slice_off && (s.tr.total == 0 || (s.tr.col && s.tr.src && s.val_tr)), "psm: factor %d has no transposed pattern", k);
-            SN_CHECK_ARG(s.fwd.total == 0 || (s.grad_packed && s.grad_vals), "psm_backward: factor %d has no gradient buffer", k);
+            SN_CHECK_ARG(!any_grad || s.fwd.total == 0 || (s.grad_packed && s.grad_vals),
+                         "psm_backward: factor %d has no gradient buffer (the factor gradient buffers are all set or all NULL)", k);
         }
         if (s.rows > ch->maxdim) ch->maxdim = s.rows;
         if (s.cols > ch->maxdim) ch->maxdim = s.cols;
@@ -451,20 +473,41 @@ int sn_psm_forward(const sn_psm_factor* factors_host, int nf, const float* x, in
         if (int rc = pack_vals(factors_host[k].fwd, factors_host[k].vals, factors_host[k].val_fwd, st)) return rc;
     const size_t smem = (size_t)2 * ch.maxdim * NS * sizeof(float);
     SN_CHECK_ARG(smem <= 227 * 1024, "psm_forward: factor dimension %d does not fit in shared memory", ch.maxdim);
-    SN_SET_MAX_SMEM((int)smem, psm_fwd_kernel);
+    if (int rc = fwd_kernel_smem(smem)) return rc;
     SN_LAUNCH("psm_fwd_kernel", st, psm_fwd_kernel<<<(unsigned)((B + NS - 1) / NS), PSM_THREADS, smem, st>>>(ch, x, ldx, y, ldy, bias, B, acts));
     return 0;
 }
 
 int sn_psm_backward(const sn_psm_factor* factors_host, int nf, const float* x, int64_t ldx, const float* grad_y, int64_t ldgy,
-                    const float* acts, float* grad_bias, int64_t B, int in_dim, int out_dim, sn_stream_t stream) {
+                    const float* acts, float* grad_bias, float* grad_x, int64_t ldgx, int64_t B, int in_dim, int out_dim, sn_stream_t stream) {
     Chain ch;
-    if (int rc = make_chain(factors_host, nf, in_dim, out_dim, true, &ch)) return rc;
+    bool param_grad = false;
+    if (int rc = make_chain(factors_host, nf, in_dim, out_dim, true, &ch, &param_grad)) return rc;
     SN_CHECK_ARG(x && grad_y, "psm_backward: NULL buffer");
+    SN_CHECK_ARG(param_grad || grad_x, "psm_backward: the factor gradient buffers and grad_x are both NULL");
+    SN_CHECK_ARG(grad_x == nullptr || ldgx >= in_dim, "psm_backward: grad_x leading dimension too small (ldgx %lld < input_dim %d)",
+                 (long long)ldgx, in_dim);
     if (B <= 0) return 0;
     cudaStream_t st = snb::as_stream(stream);
     if (grad_bias)
         if (int rc = snb::colsum_accumulate(grad_y, ldgy, B, out_dim, grad_bias, st)) return rc;
+    if (!param_grad) {
+        // grad_x only: the forward chain of the transposed factors in reverse order, S_{n-1}^T .. S_0^T applied to grad_y
+        Chain ct = ch;
+        ct.in_dim = out_dim;
+        ct.out_dim = in_dim;
+        for (int j = 0; j < nf; ++j) {
+            const Factor& F = ch.f[nf - 1 - j];
+            ct.f[j] = Factor{F.cols, F.rows, F.tr, F.fwd, nullptr};
+            if (int rc = pack_vals(factors_host[nf - 1 - j].tr, factors_host[nf - 1 - j].vals, factors_host[nf - 1 - j].val_tr, st)) return rc;
+        }
+        const size_t smem = (size_t)2 * ct.maxdim * NS * sizeof(float);
+        SN_CHECK_ARG(smem <= 227 * 1024, "psm_backward: factor dimension %d does not fit in shared memory", ct.maxdim);
+        if (int rc = fwd_kernel_smem(smem)) return rc;
+        SN_LAUNCH("psm_fwd_kernel", st, psm_fwd_kernel<<<(unsigned)((B + NS - 1) / NS), PSM_THREADS, smem, st>>>(ct, grad_y, ldgy, grad_x, ldgx, nullptr, B,
+                                                                                                            nullptr));
+        return 0;
+    }
     for (int k = 0; k < nf; ++k) {
         const sn_psm_factor& f = factors_host[k];
         if (int rc = pack_vals(f.fwd, f.vals, f.val_fwd, st)) return rc;
@@ -474,13 +517,25 @@ int sn_psm_backward(const sn_psm_factor* factors_host, int nf, const float* x, i
     if (acts != nullptr) {
         const size_t smem = (size_t)2 * ch.maxdim * NS * sizeof(float);
         SN_CHECK_ARG(smem <= 227 * 1024, "psm_backward: factor dimension %d does not fit in shared memory", ch.maxdim);
-        SN_SET_MAX_SMEM((int)smem, psm_bwd_acts_kernel);
-        SN_LAUNCH("psm_bwd_acts_kernel", st, psm_bwd_acts_kernel<<<(unsigned)((B + NS - 1) / NS), PSM_THREADS, smem, st>>>(ch, x, ldx, grad_y, ldgy, B, acts));
+        const unsigned grid = (unsigned)((B + NS - 1) / NS);
+        if (grad_x != nullptr) {
+            SN_SET_MAX_SMEM((int)smem, psm_bwd_acts_kernel<true>);
+            SN_LAUNCH("psm_bwd_acts_kernel<gx>", st, psm_bwd_acts_kernel<true><<<grid, PSM_THREADS, smem, st>>>(ch, x, ldx, grad_y, ldgy, B, acts, grad_x, ldgx));
+        } else {
+            SN_SET_MAX_SMEM((int)smem, psm_bwd_acts_kernel<false>);
+            SN_LAUNCH("psm_bwd_acts_kernel", st, psm_bwd_acts_kernel<false><<<grid, PSM_THREADS, smem, st>>>(ch, x, ldx, grad_y, ldgy, B, acts, nullptr, 0));
+        }
     } else {
         const size_t smem = (size_t)3 * ch.maxdim * NS * sizeof(float);
         SN_CHECK_ARG(smem <= 227 * 1024, "psm_backward: factor dimension %d does not fit in shared memory", ch.maxdim);
-        SN_SET_MAX_SMEM((int)smem, psm_bwd_kernel);
-        SN_LAUNCH("psm_bwd_kernel", st, psm_bwd_kernel<<<(unsigned)((B + NS - 1) / NS), PSM_THREADS, smem, st>>>(ch, x, ldx, grad_y, ldgy, B));
+        const unsigned grid = (unsigned)((B + NS - 1) / NS);
+        if (grad_x != nullptr) {
+            SN_SET_MAX_SMEM((int)smem, psm_bwd_kernel<true>);
+            SN_LAUNCH("psm_bwd_kernel<gx>", st, psm_bwd_kernel<true><<<grid, PSM_THREADS, smem, st>>>(ch, x, ldx, grad_y, ldgy, B, grad_x, ldgx));
+        } else {
+            SN_SET_MAX_SMEM((int)smem, psm_bwd_kernel<false>);
+            SN_LAUNCH("psm_bwd_kernel", st, psm_bwd_kernel<false><<<grid, PSM_THREADS, smem, st>>>(ch, x, ldx, grad_y, ldgy, B, nullptr, 0));
+        }
     }
     for (int k = 0; k < nf; ++k) {
         const sn_psm_factor& f = factors_host[k];

@@ -19,7 +19,9 @@ from structurednets_b200.layers.structured_layer import StructuredLayer
 
 
 class _HMatFunction(torch.autograd.Function):
-    """Leaf-by-leaf CUDA-core kernels (csrc/hmat.cu: sn_hmat_forward / sn_hmat_backward); kept for matrices too large to densify."""
+    """Leaf-by-leaf CUDA-core kernels (csrc/hmat.cu: sn_hmat_forward / sn_hmat_backward); kept for matrices too large to densify.
+    ``anchor`` is passed when some parameter takes a gradient; a backward that only returns ``grad_x`` leaves the flat gradient
+    buffer alone."""
 
     @staticmethod
     def forward(ctx, U, anchor, layer):
@@ -32,6 +34,7 @@ class _HMatFunction(torch.autograd.Function):
                                         layer.output_dim, _lib.stream_ptr())
         _lib.check(rc, "sn_hmat_forward")
         ctx.layer = layer
+        ctx.param_grad = anchor is not None
         ctx.save_for_backward(U, table)
         return y
 
@@ -39,17 +42,16 @@ class _HMatFunction(torch.autograd.Function):
     def backward(ctx, grad_y):
         layer = ctx.layer
         U, table = ctx.saved_tensors
-        if ctx.needs_input_grad[0]:
-            raise RuntimeError("HMatLayer: the leaf-by-leaf kernels do not return the gradient w.r.t. the input features; the dense-block "
-                               "path (default up to 2^26 matrix elements) does")
         grad_y = grad_y.contiguous().float()
-        g = layer._prepare_grad_accumulation()
-        gb = g[:layer.output_dim] if (layer.use_bias and layer.bias.requires_grad) else None
+        grad_x = torch.empty_like(U) if ctx.needs_input_grad[0] else None
+        g = layer._prepare_grad_accumulation() if ctx.param_grad else None
+        gb = g[:layer.output_dim] if (g is not None and layer.use_bias and layer.bias.requires_grad) else None
         rc = _lib.lib().sn_hmat_backward(_lib.ptr(table), layer._nleaves, _lib.ptr(layer.flat_parameters()), _lib.ptr(U), U.stride(0),
-                                         _lib.ptr(grad_y), grad_y.stride(0), _lib.ptr(g), _lib.ptr(gb), U.shape[0], layer.input_dim,
-                                         layer.output_dim, _lib.stream_ptr())
+                                         _lib.ptr(grad_y), grad_y.stride(0), _lib.ptr(g), _lib.ptr(gb), _lib.ptr(grad_x),
+                                         grad_x.stride(0) if grad_x is not None else 0, U.shape[0], layer.input_dim, layer.output_dim,
+                                         _lib.stream_ptr())
         _lib.check(rc, "sn_hmat_backward")
-        return None, None, None
+        return grad_x, None, None
 
 
 class _HMatDenseFunction(torch.autograd.Function):
@@ -274,6 +276,9 @@ class HMatLayer(FlatParamsMixin, StructuredLayer):
             anchor = torch.zeros(1, device=U.device, requires_grad=True)
             self.__dict__["_dev_anchor"] = anchor
         needs = torch.is_grad_enabled() and self._nleaves > 0
+        if fn is _HMatFunction:
+            # the leaf path computes parameter gradients only when some parameter takes one (SSSLayer decides the same way)
+            needs = needs and any(p.requires_grad for p in self._flat_param_list())
         return fn.apply(U, anchor if needs else None, self)
 
     def get_nb_parameters(self) -> int:

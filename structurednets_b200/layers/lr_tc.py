@@ -8,6 +8,7 @@ Stated tolerance (tests/test_lr_tc_gpu.py): 2e-2 relative to the largest entry, 
 import torch
 
 from structurednets_b200 import _lib
+from structurednets_b200.layers import dense_bf16 as D
 
 
 def _bf16_params(layer):
@@ -51,8 +52,6 @@ class _LRFunctionBF16(torch.autograd.Function):
     def backward(ctx, grad_y):
         layer = ctx.layer
         U, hidden = ctx.saved_tensors
-        if ctx.needs_input_grad[0]:
-            raise RuntimeError("LRLayer (bf16 path): gradient w.r.t. the input features is not implemented; use float32 features")
         B = U.shape[0]
         out_dim, rank = layer.left_lr.shape
         in_dim = layer.right_lr.shape[1]
@@ -63,19 +62,27 @@ class _LRFunctionBF16(torch.autograd.Function):
             buf = torch.empty((B, ldg), dtype=torch.bfloat16, device=U.device)
             buf[:, :out_dim] = gy
             gy = buf[:, :out_dim]
-        layer._prepare_grad_accumulation()
+        if any(p.requires_grad for p in layer._flat_param_list()):   # a frozen layer never allocates the flat gradient buffer
+            layer._prepare_grad_accumulation()
         ldt = (B + 7) // 8 * 8
         mk = lambda rows: torch.empty((rows, ldt), dtype=torch.bfloat16, device=U.device)
         ghid = torch.empty((B, rank), dtype=torch.bfloat16, device=U.device)
-        gyt, ht, ght, xt = mk(out_dim), mk(rank), mk(rank), mk(in_dim)
         gl = layer.left_lr.grad if layer.left_lr.requires_grad else None
         gr = layer.right_lr.grad if layer.right_lr.requires_grad else None
+        # transpose scratch of the dL / dR GEMMs, only for the factors that take a gradient
+        gyt, ht = (mk(out_dim), mk(rank)) if gl is not None else (None, None)
+        ght, xt = (mk(rank), mk(in_dim)) if gr is not None else (None, None)
         gb = layer.bias.grad if (layer.use_bias and layer.bias.requires_grad) else None
-        rc = _lib.lib().sn_lr_tc_backward(_lib.ptr(U), U.stride(0), _lib.ptr(gy), gy.stride(0), _lib.ptr(P["Lt"]), P["lt_ld"], _lib.ptr(hidden),
-                                          _lib.ptr(ghid), _lib.ptr(gyt), _lib.ptr(ht), _lib.ptr(ght), _lib.ptr(xt), ldt, _lib.ptr(gl), _lib.ptr(gr),
-                                          _lib.ptr(gb), B, in_dim, out_dim, rank, _lib.stream_ptr())
+        grad_x = rt = None
+        if ctx.needs_input_grad[0]:   # grad_x = ghid R, bf16 like the features (rows padded to 16 bytes for the GEMM's stores)
+            grad_x = D.empty_rows(B, in_dim, U.device)
+            rt = torch.empty((in_dim, rank), dtype=torch.bfloat16, device=U.device)
+        rc = _lib.lib().sn_lr_tc_backward(_lib.ptr(U), U.stride(0), _lib.ptr(gy), gy.stride(0), _lib.ptr(P["Lt"]), P["lt_ld"], _lib.ptr(P["R"]),
+                                          _lib.ptr(hidden), _lib.ptr(ghid), _lib.ptr(gyt), _lib.ptr(ht), _lib.ptr(ght), _lib.ptr(xt), ldt, _lib.ptr(rt),
+                                          _lib.ptr(gl), _lib.ptr(gr), _lib.ptr(gb), _lib.ptr(grad_x), grad_x.stride(0) if grad_x is not None else 0,
+                                          B, in_dim, out_dim, rank, _lib.stream_ptr())
         _lib.check(rc, "sn_lr_tc_backward")
-        return None, None, None
+        return grad_x, None, None
 
 
 def lr_forward_bf16(layer, U, anchor):

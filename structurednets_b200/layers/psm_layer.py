@@ -195,7 +195,7 @@ def _factor_array(patterns, params, gvals):
             e.rowmap, e.slice_off, e.col, e.src = d["rowmap"].data_ptr(), d["slice_off"].data_ptr(), d["col"].data_ptr(), d["src"].data_ptr()
         f.vals = p._values().data_ptr()
         f.val_fwd, f.val_tr = pat["fwd"]["val"].data_ptr(), pat["tr"]["val"].data_ptr()
-        f.grad_packed = pat["grad_packed"].data_ptr()
+        f.grad_packed = pat["grad_packed"].data_ptr() if gvals is not None else None
         f.grad_vals = gvals[k].data_ptr() if gvals is not None else None
     return arr
 
@@ -226,19 +226,22 @@ class _PSMFunction(torch.autograd.Function):
         U, acts, *factors = ctx.saved_tensors
         acts = acts if ctx.has_acts else None
         layer = ctx.layer
-        if ctx.needs_input_grad[0]:
-            raise RuntimeError("PSMLayer: the sparse-chain kernels do not return the gradient w.r.t. the input features; the dense-product "
-                               "path does (SNB200_PSM_PATH=dense, or any batch >= 1024)")
         grad_y = grad_y.contiguous().float()
-        gvals = [torch.zeros(p._nnz(), dtype=torch.float32, device=U.device) for p in factors]
-        gbias = torch.zeros(layer.output_dim, dtype=torch.float32, device=U.device) if ctx.has_bias else None
+        grad_x = torch.empty_like(U) if ctx.needs_input_grad[0] else None
+        # the factor gradients are computed when a factor takes one (or when nothing else would run: a bias-only backward)
+        param_grad = any(ctx.needs_input_grad[3:]) or grad_x is None
+        gvals = [torch.zeros(p._nnz(), dtype=torch.float32, device=U.device) for p in factors] if param_grad else None
+        # (without grad_x, param_grad holds and the bias gradient is formed as it always was)
+        gbias = torch.zeros(layer.output_dim, dtype=torch.float32, device=U.device) if ctx.has_bias and (param_grad or ctx.needs_input_grad[1]) else None
         arr = _factor_array(ctx.patterns, factors, gvals)
         rc = _lib.lib().sn_psm_backward(arr, len(factors), _lib.ptr(U), U.stride(0), _lib.ptr(grad_y), grad_y.stride(0), _lib.ptr(acts), _lib.ptr(gbias),
-                                        U.shape[0], layer.input_dim, layer.output_dim, _lib.stream_ptr())
+                                        _lib.ptr(grad_x), grad_x.stride(0) if grad_x is not None else 0, U.shape[0], layer.input_dim,
+                                        layer.output_dim, _lib.stream_ptr())
         _lib.check(rc, "sn_psm_backward")
         # sparse gradients on the parameters' own (uncoalesced) pattern, like autograd's to_dense backward
-        gf = [torch.sparse_coo_tensor(p._indices(), g, p.shape) for p, g in zip(factors, gvals)]
-        return (None, gbias, None, *gf)
+        gf = [torch.sparse_coo_tensor(p._indices(), g, p.shape) if need else None
+              for p, g, need in zip(factors, gvals or [None] * len(factors), ctx.needs_input_grad[3:])]
+        return (grad_x, gbias, None, *gf)
 
 
 class PSMLayer(StructuredLayer):
