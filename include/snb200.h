@@ -13,7 +13,10 @@
  *   - every kernel is enqueued on `stream` (a cudaStream_t passed as void*);
  *   - return value 0 = ok, non-zero = error, message in sn_last_error_string() (thread local);
  *   - matrices are row-major; "ld" arguments are row strides in elements;
- *   - gradients are ACCUMULATED (+=) into grad buffers, like torch autograd does.
+ *   - gradients are ACCUMULATED (+=) into grad buffers, like torch autograd does;
+ *   - an empty batch (B == 0) is a no-op that returns 0: every entry that takes a batch size checks its plan and parameter
+ *     arguments, then returns before it looks at any batch buffer (features, outputs, their gradients, activations and scratch
+ *     sized by B), which may then be NULL or point anywhere.  Nothing is written, accumulated gradients included.
  */
 #ifndef SNB200_H
 #define SNB200_H

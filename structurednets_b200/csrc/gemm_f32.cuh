@@ -103,6 +103,7 @@ inline int gemm_f32(bool ta, bool tb, int M, int N, int K, float alpha, const fl
                     float beta, float* C, long ldc, const float* bias, cudaStream_t stream, bool accumulate = false,
                     const int* kdev = nullptr, const int* mdev = nullptr) {
     if (M <= 0 || N <= 0) return 0;
+    if (accumulate && K <= 0) return 0;   // adds nothing (a non-accumulating K = 0 still writes bias or zeros below)
     // tensor-core path (3xTF32, csrc/gemm_tf32x3.cuh) whenever TMA can read the operands; SNB200_GEMM=simt forces the CUDA-core kernel
     {
         const char* e = getenv("SNB200_GEMM");

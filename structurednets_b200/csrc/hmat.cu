@@ -331,8 +331,9 @@ extern "C" {
 // params: flat parameter buffer holding left_lr (rows x k) and right_lr (k x cols) of every leaf at those offsets.
 int sn_hmat_forward(const int32_t* leaves, int nleaves, const float* params, const float* x, int64_t ldx, float* y, int64_t ldy,
                     const float* bias, int64_t B, int in_dim, int out_dim, sn_stream_t stream) {
-    SN_CHECK_ARG(params && x && y && (leaves || nleaves == 0), "hmat_forward: NULL buffer");
+    SN_CHECK_ARG(params && (leaves || nleaves == 0), "hmat_forward: NULL buffer");
     if (B <= 0) return 0;
+    SN_CHECK_ARG(x && y, "hmat_forward: NULL buffer");
     const int rc = hm_launch_fwd<false>(reinterpret_cast<const Leaf*>(leaves), nleaves, params, x, ldx, y, ldy, bias, B, in_dim, out_dim,
                                         snb::as_stream(stream));
     if (rc < 0) {
@@ -347,11 +348,12 @@ int sn_hmat_forward(const int32_t* leaves, int nleaves, const float* params, con
 int sn_hmat_backward(const int32_t* leaves, int nleaves, const float* params, const float* x, int64_t ldx, const float* grad_y,
                      int64_t ldgy, float* grad_params, float* grad_bias, float* grad_x, int64_t ldgx, int64_t B, int in_dim, int out_dim,
                      sn_stream_t stream) {
-    SN_CHECK_ARG(params && x && grad_y && (leaves || nleaves == 0), "hmat_backward: NULL buffer");
+    SN_CHECK_ARG(params && (leaves || nleaves == 0), "hmat_backward: NULL buffer");
+    if (B <= 0) return 0;
+    SN_CHECK_ARG(x && grad_y, "hmat_backward: NULL buffer");
     SN_CHECK_ARG(grad_params || grad_x, "hmat_backward: grad_params and grad_x are both NULL");
     SN_CHECK_ARG(grad_x == nullptr || ldgx >= in_dim, "hmat_backward: grad_x leading dimension too small (ldgx %lld < in_dim %d)",
                  (long long)ldgx, in_dim);
-    if (B <= 0) return 0;
     cudaStream_t st = snb::as_stream(stream);
     const Leaf* lv = reinterpret_cast<const Leaf*>(leaves);
     if (grad_bias)

@@ -376,12 +376,16 @@ int sn_ldr_backward(int n, int r, const float* dW, const int32_t* A_slot, int A_
 // y[B x n_out] = x[B x n_in] W^T + bias  and  dW[n_out x n_in] += gy^T x ; plain fp32 GEMMs shared by LDR and TL.
 int sn_dense_apply(const float* W, int n_out, int n_in, const float* x, int64_t ldx, float* y, int64_t ldy, const float* bias,
                    int64_t B, sn_stream_t stream) {
-    SN_CHECK_ARG(W && x && y, "dense_apply: NULL buffer");
+    SN_CHECK_ARG(W, "dense_apply: NULL buffer");
+    if (B <= 0) return 0;
+    SN_CHECK_ARG(x && y, "dense_apply: NULL buffer");
     return snb::gemm_f32(false, true, (int)B, n_out, n_in, 1.f, x, ldx, W, n_in, 0.f, y, ldy, bias, snb::as_stream(stream));
 }
 int sn_dense_weight_grad(const float* x, int64_t ldx, const float* gy, int64_t ldgy, float* dW, int n_out, int n_in, float* grad_bias,
                          int64_t B, sn_stream_t stream) {
-    SN_CHECK_ARG(x && gy && dW, "dense_weight_grad: NULL buffer");
+    SN_CHECK_ARG(dW, "dense_weight_grad: NULL buffer");
+    if (B <= 0) return 0;
+    SN_CHECK_ARG(x && gy, "dense_weight_grad: NULL buffer");
     cudaStream_t st = snb::as_stream(stream);
     if (grad_bias)
         if (int rc = snb::colsum_accumulate(gy, ldgy, B, n_out, grad_bias, st)) return rc;
@@ -390,7 +394,9 @@ int sn_dense_weight_grad(const float* x, int64_t ldx, const float* gy, int64_t l
 
 // grad_x[B x n_in] = grad_y[B x n_out] W  (the gradient w.r.t. the input features of every layer that materialises W)
 int sn_dense_input_grad(const float* W, int n_out, int n_in, const float* gy, int64_t ldgy, float* gx, int64_t ldgx, int64_t B, sn_stream_t stream) {
-    SN_CHECK_ARG(W && gy && gx, "dense_input_grad: NULL buffer");
+    SN_CHECK_ARG(W, "dense_input_grad: NULL buffer");
+    if (B <= 0) return 0;
+    SN_CHECK_ARG(gy && gx, "dense_input_grad: NULL buffer");
     return snb::gemm_f32(false, false, (int)B, n_in, n_out, 1.f, gy, ldgy, W, n_in, 0.f, gx, ldgx, nullptr, snb::as_stream(stream));
 }
 

@@ -9,10 +9,11 @@ extern "C" {
 
 int sn_lr_forward_f32(const float* x, int64_t ldx, const float* left, const float* right, const float* bias, float* hidden,
                       float* y, int64_t ldy, int64_t B, int in_dim, int out_dim, int rank, sn_stream_t stream) {
-    SN_CHECK_ARG(x && left && right && hidden && y, "lr_forward: NULL buffer");
+    SN_CHECK_ARG(left && right, "lr_forward: NULL buffer");
     SN_CHECK_ARG(in_dim > 0 && out_dim > 0 && rank >= 0 && B >= 0, "lr_forward: bad dims");
-    cudaStream_t s = snb::as_stream(stream);
     if (B == 0) return 0;
+    SN_CHECK_ARG(x && hidden && y, "lr_forward: NULL buffer");
+    cudaStream_t s = snb::as_stream(stream);
     // h = x R^T : (B x in) (r x in)^T
     if (int rc = snb::gemm_f32(false, true, (int)B, rank, in_dim, 1.f, x, ldx, right, in_dim, 0.f, hidden, rank, nullptr, s)) return rc;
     // y = h L^T + b : (B x r) (out x r)^T
@@ -22,9 +23,10 @@ int sn_lr_forward_f32(const float* x, int64_t ldx, const float* left, const floa
 int sn_lr_backward_f32(const float* x, int64_t ldx, const float* grad_y, int64_t ldgy, const float* left, const float* right,
                        const float* hidden, float* grad_hidden_ws, float* grad_left, float* grad_right, float* grad_bias,
                        float* grad_x, int64_t ldgx, int64_t B, int in_dim, int out_dim, int rank, sn_stream_t stream) {
-    SN_CHECK_ARG(x && grad_y && left && right && hidden && grad_hidden_ws, "lr_backward: NULL buffer");
+    SN_CHECK_ARG(left && right, "lr_backward: NULL buffer");
+    if (B <= 0) return 0;
+    SN_CHECK_ARG(x && grad_y && hidden && grad_hidden_ws, "lr_backward: NULL buffer");
     cudaStream_t s = snb::as_stream(stream);
-    if (B == 0) return 0;
     // gh = gy L : (B x out) (out x r)
     if (int rc = snb::gemm_f32(false, false, (int)B, rank, out_dim, 1.f, grad_y, ldgy, left, rank, 0.f, grad_hidden_ws, rank, nullptr, s)) return rc;
     if (grad_left)   // dL += gy^T h : (out x B) (B x r)

@@ -249,9 +249,10 @@ int sn_lr_tc_cast_params(const float* left, const float* right, void* left_bf16,
 // x (B x in) bf16, hidden (B x rank) bf16 [written], y (B x out) bf16 [written]; all row pitches multiples of 8 elements
 int sn_lr_tc_forward(const void* x, int64_t ldx, const void* left_bf16, const void* right_bf16, const float* bias, void* hidden, void* y,
                      int64_t ldy, int64_t B, int in_dim, int out_dim, int rank, sn_stream_t stream) {
-    SN_CHECK_ARG(x && left_bf16 && right_bf16 && hidden && y, "lr_tc_forward: NULL buffer");
+    SN_CHECK_ARG(left_bf16 && right_bf16, "lr_tc_forward: NULL buffer");
     SN_CHECK_ARG(rank % 8 == 0 && rank >= 8, "lr_tc_forward: the tensor-core path needs rank %% 8 == 0 (got %d)", rank);
     if (B <= 0) return 0;
+    SN_CHECK_ARG(x && hidden && y, "lr_tc_forward: NULL buffer");
     cudaStream_t st = snb::as_stream(stream);
     using namespace snb::tc;
     {
@@ -285,14 +286,15 @@ int sn_lr_tc_backward(const void* x, int64_t ldx, const void* grad_y, int64_t ld
                       const void* right_bf16, const void* hidden, void* ghid, void* gyt, void* ht, void* ght, void* xt, int64_t ldt,
                       void* right_t, float* grad_left, float* grad_right, float* grad_bias, void* grad_x, int64_t ldgx, int64_t B,
                       int in_dim, int out_dim, int rank, sn_stream_t stream) {
-    SN_CHECK_ARG(x && grad_y && left_t_bf16 && hidden && ghid, "lr_tc_backward: NULL buffer");
+    SN_CHECK_ARG(left_t_bf16, "lr_tc_backward: NULL buffer");
+    if (B <= 0) return 0;
+    SN_CHECK_ARG(x && grad_y && hidden && ghid, "lr_tc_backward: NULL buffer");
     SN_CHECK_ARG((grad_left == nullptr || (gyt && ht)) && (grad_right == nullptr || (ght && xt)), "lr_tc_backward: NULL transpose scratch");
     SN_CHECK_ARG(ldt >= B && ldt % 8 == 0, "lr_tc_backward: ldt must be B rounded up to a multiple of 8");
     SN_CHECK_ARG(grad_x == nullptr || (right_bf16 && right_t), "lr_tc_backward: grad_x needs right_bf16 and the right_t scratch");
     SN_CHECK_ARG(grad_x == nullptr || ldgx >= in_dim, "lr_tc_backward: grad_x leading dimension too small (ldgx %lld < in_dim %d)",
                  (long long)ldgx, in_dim);
     SN_CHECK_ARG(grad_x == nullptr || ldgx % 8 == 0, "lr_tc_backward: grad_x leading dimension %lld is not a multiple of 8", (long long)ldgx);
-    if (B <= 0) return 0;
     cudaStream_t st = snb::as_stream(stream);
     using namespace snb::tc;
     // side stream: bias gradient and dL (they need grad_y and the hidden activations only); main stream: gh, then dR

@@ -466,8 +466,8 @@ int sn_psm_forward(const sn_psm_factor* factors_host, int nf, const float* x, in
                    float* acts, int64_t B, int in_dim, int out_dim, sn_stream_t stream) {
     Chain ch;
     if (int rc = make_chain(factors_host, nf, in_dim, out_dim, false, &ch)) return rc;
-    SN_CHECK_ARG(x && y, "psm_forward: NULL buffer");
     if (B <= 0) return 0;
+    SN_CHECK_ARG(x && y, "psm_forward: NULL buffer");
     cudaStream_t st = snb::as_stream(stream);
     for (int k = 0; k < nf; ++k)
         if (int rc = pack_vals(factors_host[k].fwd, factors_host[k].vals, factors_host[k].val_fwd, st)) return rc;
@@ -483,11 +483,11 @@ int sn_psm_backward(const sn_psm_factor* factors_host, int nf, const float* x, i
     Chain ch;
     bool param_grad = false;
     if (int rc = make_chain(factors_host, nf, in_dim, out_dim, true, &ch, &param_grad)) return rc;
+    if (B <= 0) return 0;
     SN_CHECK_ARG(x && grad_y, "psm_backward: NULL buffer");
     SN_CHECK_ARG(param_grad || grad_x, "psm_backward: the factor gradient buffers and grad_x are both NULL");
     SN_CHECK_ARG(grad_x == nullptr || ldgx >= in_dim, "psm_backward: grad_x leading dimension too small (ldgx %lld < input_dim %d)",
                  (long long)ldgx, in_dim);
-    if (B <= 0) return 0;
     cudaStream_t st = snb::as_stream(stream);
     if (grad_bias)
         if (int rc = snb::colsum_accumulate(grad_y, ldgy, B, out_dim, grad_bias, st)) return rc;
@@ -560,8 +560,9 @@ size_t sn_psm_dense_backward_floats(const sn_psm_dense_factor* f, int nf, int ou
 int sn_psm_dense_forward(const sn_psm_dense_factor* f, int nf, const float* x, int64_t ldx, float* y, int64_t ldy, const float* bias,
                          float* prefix, int64_t B, int in_dim, int out_dim, sn_stream_t stream) {
     if (int rc = check_dense_chain(f, nf, in_dim, out_dim)) return rc;
-    SN_CHECK_ARG(x && y && prefix, "psm_dense_forward: NULL buffer");
+    SN_CHECK_ARG(prefix, "psm_dense_forward: NULL buffer");
     if (B <= 0) return 0;
+    SN_CHECK_ARG(x && y, "psm_dense_forward: NULL buffer");
     cudaStream_t st = snb::as_stream(stream);
     const float* wt = nullptr;
     if (int rc = build_prefix(f, nf, prefix, out_dim, &wt, st)) return rc;
@@ -572,8 +573,9 @@ int sn_psm_dense_forward(const sn_psm_dense_factor* f, int nf, const float* x, i
 int sn_psm_dense_input_grad(const sn_psm_dense_factor* f, int nf, const float* prefix, const float* grad_y, int64_t ldgy, float* grad_x,
                             int64_t ldgx, int64_t B, int in_dim, int out_dim, sn_stream_t stream) {
     if (int rc = check_dense_chain(f, nf, in_dim, out_dim)) return rc;
-    SN_CHECK_ARG(prefix && grad_y && grad_x, "psm_dense_input_grad: NULL buffer");
+    SN_CHECK_ARG(prefix, "psm_dense_input_grad: NULL buffer");
     if (B <= 0) return 0;
+    SN_CHECK_ARG(grad_y && grad_x, "psm_dense_input_grad: NULL buffer");
     size_t off = 0;
     for (int k = 0; k + 1 < nf; ++k) off += (size_t)f[k].cols * out_dim;
     return snb::gemm_f32(false, true, (int)B, in_dim, out_dim, 1.f, grad_y, ldgy, prefix + off, out_dim, 0.f, grad_x, ldgx, nullptr, snb::as_stream(stream));
@@ -582,8 +584,9 @@ int sn_psm_dense_input_grad(const sn_psm_dense_factor* f, int nf, const float* p
 int sn_psm_dense_backward(const sn_psm_dense_factor* f, int nf, const float* x, int64_t ldx, const float* grad_y, int64_t ldgy,
                           const float* prefix, float* work, float* grad_bias, int64_t B, int in_dim, int out_dim, sn_stream_t stream) {
     if (int rc = check_dense_chain(f, nf, in_dim, out_dim)) return rc;
-    SN_CHECK_ARG(x && grad_y && prefix && work, "psm_dense_backward: NULL buffer");
+    SN_CHECK_ARG(prefix && work, "psm_dense_backward: NULL buffer");
     if (B <= 0) return 0;
+    SN_CHECK_ARG(x && grad_y, "psm_dense_backward: NULL buffer");
     cudaStream_t st = snb::as_stream(stream);
     if (grad_bias)
         if (int rc = snb::colsum_accumulate(grad_y, ldgy, B, out_dim, grad_bias, st)) return rc;
@@ -600,8 +603,9 @@ int sn_psm_dense_forward_bf16(const sn_psm_dense_factor* f, int nf, const void* 
                               float* prefix, void* wb, int64_t ldwb, void* wtb, int64_t ldwtb, int64_t B, int in_dim, int out_dim,
                               sn_stream_t stream) {
     if (int rc = check_dense_chain(f, nf, in_dim, out_dim)) return rc;
-    SN_CHECK_ARG(x && y && prefix && wb, "psm_dense_forward_bf16: NULL buffer");
+    SN_CHECK_ARG(prefix && wb, "psm_dense_forward_bf16: NULL buffer");
     if (B <= 0) return 0;
+    SN_CHECK_ARG(x && y, "psm_dense_forward_bf16: NULL buffer");
     const float* wt = nullptr;
     if (int rc = build_prefix(f, nf, prefix, out_dim, &wt, snb::as_stream(stream))) return rc;
     // the last prefix block is W^T [in_dim][out_dim]: its copy is W^T, its transpose W
@@ -611,8 +615,9 @@ int sn_psm_dense_forward_bf16(const sn_psm_dense_factor* f, int nf, const void* 
 int sn_psm_dense_backward_bf16(const sn_psm_dense_factor* f, int nf, const void* x, int64_t ldx, const void* grad_y, int64_t ldgy,
                                const float* prefix, float* work, float* grad_bias, int64_t B, int in_dim, int out_dim, sn_stream_t stream) {
     if (int rc = check_dense_chain(f, nf, in_dim, out_dim)) return rc;
-    SN_CHECK_ARG(x && grad_y && prefix && work, "psm_dense_backward_bf16: NULL buffer");
+    SN_CHECK_ARG(prefix && work, "psm_dense_backward_bf16: NULL buffer");
     if (B <= 0) return 0;
+    SN_CHECK_ARG(x && grad_y, "psm_dense_backward_bf16: NULL buffer");
     cudaStream_t st = snb::as_stream(stream);
     if (grad_bias)
         if (int rc = colsum_bf16((const __nv_bfloat16*)grad_y, ldgy, B, out_dim, grad_bias, st)) return rc;

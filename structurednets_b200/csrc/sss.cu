@@ -993,9 +993,10 @@ int sn_sss_pack(const sn_sss_plan* p, const float* params, float* packed, sn_str
 int sn_sss_forward(const sn_sss_plan* p, const float* packed, const float* x, int64_t ldx, float* y, int64_t ldy,
                    const float* bias, float* ckpt, int64_t B, sn_stream_t stream) {
     if (int rc = check_plan(p)) return rc;
-    SN_CHECK_ARG(packed && x && y, "sss_forward: NULL buffer");
-    SN_CHECK_ARG(ldx >= p->input_dim && ldy >= p->output_dim, "sss_forward: leading dimension too small");
+    SN_CHECK_ARG(packed, "sss_forward: NULL buffer");
     if (B <= 0) return 0;
+    SN_CHECK_ARG(x && y, "sss_forward: NULL buffer");
+    SN_CHECK_ARG(ldx >= p->input_dim && ldy >= p->output_dim, "sss_forward: leading dimension too small");
     Geom g = make_geom(p->rows_pad);
     // 16-byte cp.async path needs 16-byte aligned rows whose length is a multiple of 4 floats
     const int aligned = ((reinterpret_cast<uintptr_t>(x) & 15) == 0 && (ldx & 3) == 0 && (p->input_dim & 3) == 0) ? 1 : 0;
@@ -1019,12 +1020,13 @@ int sn_sss_backward(const sn_sss_plan* p, const float* packed, const float* x, i
                     int64_t ldgy, const float* ckpt, float* workspace, float* grad_params, float* grad_bias, float* grad_x,
                     int64_t ldgx, int64_t B, sn_stream_t stream) {
     if (int rc = check_plan(p)) return rc;
-    SN_CHECK_ARG(packed && x && grad_y && ckpt, "sss_backward: NULL buffer");
-    SN_CHECK_ARG(grad_params != nullptr || grad_x != nullptr, "sss_backward: grad_params and grad_x are both NULL (nothing to compute)");
+    SN_CHECK_ARG(packed, "sss_backward: NULL buffer");
     SN_CHECK_ARG(grad_params == nullptr || workspace != nullptr, "sss_backward: NULL workspace");
+    if (B <= 0) return 0;
+    SN_CHECK_ARG(x && grad_y && ckpt, "sss_backward: NULL buffer");
+    SN_CHECK_ARG(grad_params != nullptr || grad_x != nullptr, "sss_backward: grad_params and grad_x are both NULL (nothing to compute)");
     SN_CHECK_ARG(ldx >= p->input_dim && ldgy >= p->output_dim, "sss_backward: leading dimension too small");
     SN_CHECK_ARG(grad_x == nullptr || ldgx >= p->input_dim, "sss_backward: grad_x leading dimension too small");
-    if (B <= 0) return 0;
     cudaStream_t st = snb::as_stream(stream);
     Geom g = make_geom(p->rows_pad);
     BwdSmem sm = make_bwd_smem(*p, g, grad_x != nullptr);

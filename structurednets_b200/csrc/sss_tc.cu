@@ -3613,9 +3613,10 @@ int sn_sss_tc_build(const sn_sss_tc_plan* p, const float* params, float* coef, s
 int sn_sss_tc_forward(const sn_sss_tc_plan* p, const float* coef, const float* x, int64_t ldx, float* y, int64_t ldy, const float* bias,
                       float* rbuf, float* states, int64_t B, sn_stream_t stream) {
     if (int rc = check_tc_plan(p)) return rc;
-    SN_CHECK_ARG(coef && x && y && states, "sss_tc_forward: NULL buffer");
-    SN_CHECK_ARG(ldx >= p->input_dim && ldy >= p->output_dim, "sss_tc_forward: leading dimension too small");
+    SN_CHECK_ARG(coef, "sss_tc_forward: NULL buffer");
     if (B <= 0) return 0;
+    SN_CHECK_ARG(x && y && states, "sss_tc_forward: NULL buffer");
+    SN_CHECK_ARG(ldx >= p->input_dim && ldy >= p->output_dim, "sss_tc_forward: leading dimension too small");
     cudaStream_t st = snb::as_stream(stream);
     const float* W = coef;
     const float* SC = coef + (size_t)p->nchunks * WROWS * WCOLS;
@@ -3708,12 +3709,13 @@ int sn_sss_tc_backward(const sn_sss_tc_plan* p, const float* params, const float
                        int64_t ldgy, const float* states, float* workspace, float* grad_params, float* grad_bias, float* grad_x, int64_t ldgx,
                        int64_t B, sn_stream_t stream) {
     if (int rc = check_tc_plan(p)) return rc;
-    SN_CHECK_ARG(params && coef && x && grad_y && states && workspace, "sss_tc_backward: NULL buffer");
+    SN_CHECK_ARG(params && coef, "sss_tc_backward: NULL buffer");
+    if (B <= 0) return 0;
+    SN_CHECK_ARG(x && grad_y && states && workspace, "sss_tc_backward: NULL buffer");
     SN_CHECK_ARG(grad_params != nullptr || grad_x != nullptr, "sss_tc_backward: grad_params and grad_x are both NULL (nothing to compute)");
     SN_CHECK_ARG(ldx >= p->input_dim && ldgy >= p->output_dim, "sss_tc_backward: leading dimension too small");
     SN_CHECK_ARG((ldgy & 3) == 0 && (reinterpret_cast<uintptr_t>(grad_y) & 15) == 0, "sss_tc_backward: grad_y must be 16-byte aligned with a row pitch multiple of 4");
     SN_CHECK_ARG(grad_x == nullptr || ldgx >= p->input_dim, "sss_tc_backward: grad_x leading dimension too small");
-    if (B <= 0) return 0;
     cudaStream_t st = snb::as_stream(stream);
     const float* SC = coef + (size_t)p->nchunks * WROWS * WCOLS;
     float* L = workspace;
